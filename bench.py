@@ -2,7 +2,7 @@
 """Benchmark of the multi-particle stochastic-node hot path (BASELINE.json metric):
 particle-samples/s for the IWAE / VIMCO objective forward+backward at K=50, plus % of HBM peak.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload iwae|vimco] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload iwae|vimco] [--impl reference] [--dump-outputs DIR]
 
 One "step" = one pass of the hot path over one batch of synthetic input of config 2
 (K=50 particles, B=1024 batch columns per GPU, Z=40 latent, X=784 observed; fp32):
@@ -32,6 +32,8 @@ import sys
 import threading
 import time
 
+sys.dont_write_bytecode = True  # the benchmark writes nothing into the tree it runs from, which may be read-only
+
 ROOT = os.path.dirname(os.path.abspath(__file__))
 PKG = os.path.join(ROOT, "zhusuan-pytorch_b200")
 REF = os.path.join(ROOT, "baseline", "_ref")
@@ -41,12 +43,22 @@ VAE_DECODER_PARAMS = 40 * 500 + 500 + 500 * 500 + 500 + 500 * 784 + 784         
 VAE_ENCODER_PARAMS = 784 * 500 + 500 + 500 * 500 + 500 + 2 * (500 * 40 + 40)     # iwae.py:89-97
 FALLBACK_HBM_GBS = 6650.0
 METRIC = "particle-samples/sec for IWAE/VIMCO fwd+bwd (K=50)"
+DUMP_COLUMNS = 256  # --dump-outputs: [50, 256, 784] float32 of the likelihood gradient is 40 MB, the whole dump < 64 MB
+
+
+def positive_int(s):
+    v = int(s)
+    if v < 1:
+        raise argparse.ArgumentTypeError("must be at least 1, got %d" % v)
+    return v
 
 
 def parse_args():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=2000)
+    ap.add_argument("--steps", type=positive_int, default=2000,
+                    help="timed steps of the measurement.  --impl reference times this many steps on the host CPU "
+                         "(tens of ms each, twice over with the real reference): use a few, e.g. --steps 7")
     ap.add_argument("--warmup", type=int, default=200)
     ap.add_argument("--workload", choices=["iwae", "vimco"], default="iwae")
     ap.add_argument("--impl", choices=["b200", "reference"], default="b200")
@@ -58,7 +70,14 @@ def parse_args():
     ap.add_argument("--graph", type=int, default=1, help="replay the step from a CUDA graph (1) or launch eagerly (0)")
     ap.add_argument("--batch", type=int, default=B_COLS, help="batch columns per GPU of the headline measurement")
     ap.add_argument("--port", action="store_true", help="--impl reference: time the oracle's C port, not the reference")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one returned (rank 0: the loss and the leaves' "
+                         "gradients) as DIR/<name>.npy, float32; arrays with a batch axis keep a fixed seeded "
+                         "choice of %d batch columns" % DUMP_COLUMNS)
+    args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the b200 path")
+    return args
 
 
 def hbm_peak():
@@ -251,7 +270,7 @@ def run_reference_arm(args):
     if rank != 0:
         return
     vimco = args.workload == "vimco"
-    steps = max(1, min(args.steps, 12))
+    steps = args.steps
     warm = max(1, min(args.warmup, 3))
     use_real = os.path.isdir(os.path.join(REF, "zhusuan")) and not args.port
     if use_real:
@@ -576,8 +595,24 @@ def time_steps(torch, dist, run, steps, warm, world):
     return max(by_rank), by_rank, (t0, t1)
 
 
-def measure_api(torch, dist, zd, be, vimco, dev, B, world, rank, steps, warm, use_graph, collectives):
-    """One configuration of the product path: returns dict(ms, by_rank, launch, launches_per_step, comm)."""
+def step_outputs(torch, vimco, loss, leaves, B):
+    """What a caller of the step holds after it -- the loss and the leaves' gradients -- as float32 numpy arrays.  The
+    batch axis keeps the columns of a fixed seeded choice of DUMP_COLUMNS (all of them when B is no larger)."""
+    import numpy as np
+    cols = np.sort(np.random.RandomState(0).choice(B, min(B, DUMP_COLUMNS), replace=False))
+    idx = torch.as_tensor(cols, device=loss.device)
+    names = {"probs": "probs_grad", "a": "q_probs_grad" if vimco else "mean_grad", "b": "std_grad"}
+    out = {"loss": loss.detach().float().cpu().numpy()}
+    for key, name in names.items():
+        if key in leaves:
+            g = leaves[key].grad
+            out[name] = g.index_select(1 if key == "probs" else 0, idx).float().cpu().numpy()
+    return out
+
+
+def measure_api(torch, dist, zd, be, vimco, dev, B, world, rank, steps, warm, use_graph, collectives, keep=False):
+    """One configuration of the product path: returns dict(ms, by_rank, launch, launches_per_step, comm), and with
+    `keep` also the outputs of the last timed step (step_outputs)."""
     leaves = make_leaves(torch, vimco, dev, B, seed=1234 + rank)
     bucket = None
     comm = None
@@ -602,9 +637,16 @@ def measure_api(torch, dist, zd, be, vimco, dev, B, world, rank, steps, warm, us
                         "when dprobs is done (overlaps the latent backward), encoder segment after it"
                         % (VAE_DECODER_PARAMS, VAE_ENCODER_PARAMS)}
     step = make_api_step(torch, vimco, leaves, dev, B, world, bucket)
-    run, how, launches = capture(torch, step, dev, use_graph, count=lambda: be.launch_count)
+    last = {}
+
+    def step_kept():  # a graph replay rewrites the loss tensor (and the gradients) recorded at capture
+        last["loss"] = step()
+
+    run, how, launches = capture(torch, step_kept, dev, use_graph, count=lambda: be.launch_count)
     ms, by_rank, wall = time_steps(torch, dist, run, steps, warm, world)
     out = dict(ms=ms, by_rank=by_rank, launch=how, launches_per_step=launches, comm=comm, wall=wall, run=run)
+    if keep:
+        out["outputs"] = step_outputs(torch, vimco, last["loss"], leaves, B)
     return out
 
 
@@ -625,6 +667,7 @@ def run_b200_arm(args):
     torch.cuda.set_device(local)
     dev = torch.device("cuda", local)
     be.load()
+    torch.manual_seed(0)  # the latent noise: with the same arguments every run computes the same outputs
     pinned_to = pin_to_gpu_numa(local, local, int(os.environ.get("LOCAL_WORLD_SIZE", str(world))))
     vimco = args.workload == "vimco"
     B = int(args.batch)
@@ -647,7 +690,8 @@ def run_b200_arm(args):
         clocks.start()
 
     # ---- headline: the product path (public API, device-resident, graph replay), collectives every step when N > 1
-    head = measure_api(torch, dist, zd, be, vimco, dev, B, world, rank, args.steps, args.warmup, use_graph, True)
+    head = measure_api(torch, dist, zd, be, vimco, dev, B, world, rank, args.steps, args.warmup, use_graph, True,
+                       keep=bool(args.dump_outputs) and rank == 0)
     ms_per_step = head["ms"]
     value = world * K_PART * B / (ms_per_step * 1e-3)
     t_start, t_end = head["wall"]
@@ -776,6 +820,11 @@ def run_b200_arm(args):
         line["cpu_baseline"] = cpu_baseline_subprocess(args.workload)
     elif rank == 0:
         line["cpu_baseline"] = None
+    if rank == 0 and args.dump_outputs:
+        import numpy as np
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in head["outputs"].items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), a)
     if rank == 0:
         print(json.dumps(line))
     if world > 1 or dist.is_initialized():
