@@ -42,7 +42,7 @@ extern "C" {
 #endif
 
 /* 3: zs_allreduce_sum_peer takes (extra_src, extra_index); new: zs_allreduce_sum_nvls, zs_iw_bernoulli_fused_loss,
- *    zs_debug_set_latent_fwd.  2: device-side Philox state, handle-based host step, flags argument of the fused kernel. */
+ *    zs_debug_set_latent_fwd; later additions (compatible): zs_poisson_*, zs_iw_poisson_fused[_loss].  2: device-side Philox state, handle-based host step, flags argument of the fused kernel. */
 #define ZS_ABI_VERSION 3
 
 typedef void* zs_stream_t; /* cudaStream_t */
@@ -180,6 +180,23 @@ int zs_bernoulli_logits_logpmf_bwd(int dtype, void* dx, void* dlogits, const voi
                                    const void* logits, int logits_mode, int64_t K, int64_t M, int64_t E,
                                    zs_stream_t stream);
 
+/* ---- Poisson stochastic node ------------------------------------------------------------------------------
+ * The reference's Poisson (zhusuan/distributions/poisson.py) wraps torch.distributions.Poisson; these replace
+ * Poisson._sample (:61, torch.distributions.Poisson.sample) and Poisson._log_prob (:75) + the event sums.
+ * zs_poisson_sample: out[K,N] = Poisson(rate) counts as float values, rate mode ZS_FULL|ZS_KBCAST|ZS_SCALAR.  Knuth's
+ *   product of uniforms for rate < 10, Hormann's transformed rejection (PTRS) for rate >= 10, as ATen's CPU sampler.
+ *   Element i takes its uniforms from the Philox groups (counter i | (j << 48), j = 0, 1, ...; at most 64 groups) of
+ *   the position (seed, offset [+ rng_state]): independent of the launch geometry.  Needs K*N < 2^48.
+ *   Rates are not validated: negative or NaN rates give 0; rate must be finite.                                    */
+int zs_poisson_sample(int dtype, void* out, const void* rate, int rate_mode, int64_t K, int64_t N, uint64_t seed,
+                      uint64_t offset, void* rng_state, zs_stream_t stream);
+/* out[K,M] = sum_e ( xlogy(x, rate) - rate - lgamma(x + 1) )    (poisson.py:75, torch.distributions.Poisson.log_prob) */
+int zs_poisson_logpmf_fwd(int dtype, void* out, const void* x, int x_mode, const void* rate, int rate_mode, int64_t K,
+                          int64_t M, int64_t E, zs_stream_t stream);
+/* drate = g * (x / rate - 1); the count has no gradient.  drate may be NULL (nothing to do).                          */
+int zs_poisson_logpmf_bwd(int dtype, void* drate, const void* g, const void* x, int x_mode, const void* rate,
+                          int rate_mode, int64_t K, int64_t M, int64_t E, zs_stream_t stream);
+
 /* ---- fused latent-node kernels (zs_latent.cu) -------------------------------
  * Forward: z ~ q (Philox or injected noise), log q(z) and log p(z) under the prior, both summed over
  * E, in ONE launch: Normal._sample + Normal._log_prob twice (normal.py:89-126; the variational net's
@@ -310,6 +327,20 @@ int zs_iw_bernoulli_fused_loss(int estimator, float* loss_out, void* workspace, 
                                float* dlogp, float* dlogq, float* logpx_out, const float* probs, const float* x,
                                const float* logp_other, const float* logq, int64_t K, int64_t B, int64_t X,
                                double grad_scale, int flags, zs_stream_t stream);
+
+/* The same fused step for a POISSON likelihood over rates [K,B,X] (zhusuan/distributions/poisson.py:75 instead of
+ * bernoulli.py:84-95) with counts x[B,X]; same arguments, flags (ZS_FUSED_LOGITS excepted), workspace and results as
+ * the Bernoulli pair above, `drate` in place of `dprobs`.  log p(x_b | rate_k) = sum_x (xlogy(x, r) - r) - C_b with
+ * C_b = sum_x lgamma(x + 1), formed once per column.  Only the fixed-geometry box kernel takes it: X in {128, 256,
+ * 512, 784, 1024}, K <= 50, f32, 16-byte aligned rate / drate / x; otherwise ZS_ERR_UNSUPPORTED / ZS_ERR_ALIGN and
+ * the caller composes zs_poisson_logpmf_fwd -> zs_iw_objective -> zs_poisson_logpmf_bwd.                        */
+int zs_iw_poisson_fused(int estimator, float* cost, float* drate, float* dlogp, float* dlogq, float* logpx_out,
+                        const float* rate, const float* x, const float* logp_other, const float* logq, int64_t K,
+                        int64_t B, int64_t X, double grad_scale, int flags, zs_stream_t stream);
+int zs_iw_poisson_fused_loss(int estimator, float* loss_out, void* workspace, float* cost, float* drate, float* dlogp,
+                             float* dlogq, float* logpx_out, const float* rate, const float* x,
+                             const float* logp_other, const float* logq, int64_t K, int64_t B, int64_t X,
+                             double grad_scale, int flags, zs_stream_t stream);
 
 /* Debug hooks.  zs_debug_set_trace: device buffer (grid*40 int64) that the generic box / ring kernels fill with
  * clock64() phase timestamps of each CTA's first 8 columns; NULL (default) disables tracing.

@@ -1,5 +1,6 @@
 // Fused resident-column kernel: Bernoulli likelihood log-pmf + importance-weighted objective
-// (SGVB or VIMCO), forward AND backward, one launch, probs read from HBM once.
+// (SGVB or VIMCO), forward AND backward, one launch, probs read from HBM once.  The fixed-geometry box kernel also
+// has a Poisson-likelihood instantiation (k_iw_poisson_boxf: rates [K,B,X], counts x [B,X]).
 //
 // Replaces, for a Bernoulli likelihood node under ImportanceWeightedObjective (reference file:line):
 //   Bernoulli._log_prob            zhusuan/distributions/bernoulli.py:84-95   (fwd + autograd bwd)
@@ -1119,6 +1120,99 @@ __device__ __forceinline__ void boxf_phase_b(uint32_t bs, uint32_t bs_addr, uint
     }
 }
 
+// Poisson likelihood (zhusuan/distributions/poisson.py:75): log p(x | r) = sum_x (xlogy(x, r) - r) - C_b.  The stager
+// stages the raw counts and C_b = sum_x lgamma(x + 1) once per column (it shifts every log-weight of the column by the
+// same amount: no weight and no gradient depends on it); the row warps add x log2(r) -- skipped where x == 0, which is
+// most elements of count data -- and r separately.
+// log(k!) for k < 32: counts are mostly small integers, and lgammaf on the stager's single warp (a long dependent
+// chain per element) otherwise sets the column period
+__constant__ float c_log_factorial[32] = {
+    0.000000000e+00f, 0.000000000e+00f, 6.931471806e-01f, 1.791759469e+00f,
+    3.178053830e+00f, 4.787491743e+00f, 6.579251212e+00f, 8.525161361e+00f,
+    1.060460290e+01f, 1.280182748e+01f, 1.510441257e+01f, 1.750230785e+01f,
+    1.998721450e+01f, 2.255216385e+01f, 2.519122118e+01f, 2.789927138e+01f,
+    3.067186011e+01f, 3.350507345e+01f, 3.639544521e+01f, 3.933988419e+01f,
+    4.233561646e+01f, 4.538013890e+01f, 4.847118135e+01f, 5.160667557e+01f,
+    5.478472940e+01f, 5.800360522e+01f, 6.126170176e+01f, 6.455753863e+01f,
+    6.788974314e+01f, 7.125703897e+01f, 7.465823635e+01f, 7.809222355e+01f};
+__device__ __forceinline__ float lgamma1p_count(float v) {
+    return (v >= 0.f && v < 32.f && v == truncf(v)) ? c_log_factorial[(int)v] : lgammaf(v + 1.f);
+}
+__device__ __forceinline__ void stage_x_poisson(float* s_xrow, int* s_cb, const float* __restrict__ xrow, int X4, int lane) {
+    const float4* src = reinterpret_cast<const float4*>(xrow);
+    float4* dst = reinterpret_cast<float4*>(s_xrow);
+    float c = 0.f;
+    for (int v = lane; v < X4; v += 32) {
+        const float4 t = __ldg(src + v);
+        dst[v] = t;
+        c += (lgamma1p_count(t.x) + lgamma1p_count(t.y)) + (lgamma1p_count(t.z) + lgamma1p_count(t.w));
+    }
+    c = warp_sum(c);
+    if (lane == 0) *s_cb = __float_as_int(c);
+}
+__device__ __forceinline__ float xlog2(float x, float r) { return x == 0.f ? 0.f : x * fast_log2(r); }
+
+template <int INNER4, int NBOX>
+__device__ __forceinline__ void boxf_phase_a_poisson(BoxCursor& cur, uint32_t slots_u, uint32_t slot_bytes, uint32_t nslot,
+                                                     uint32_t full_u, uint32_t empty_u, uint32_t row_a, uint32_t row_b,
+                                                     uint32_t x_u, int lane, bool release, float& acc_a, float& acc_b,
+                                                     float& rsum_a, float& rsum_b) {
+    constexpr int VIT = (INNER4 + 31) / 32;
+#pragma unroll
+    for (int q = 0; q < NBOX; ++q) {
+        mbar_wait_u32(full_u + cur.slot * 8, cur.parity);
+#pragma unroll
+        for (int i = 0; i < VIT; ++i) {
+            if ((i + 1) * 32 <= INNER4 || lane + 32 * i < INNER4) {
+                const uint32_t o = (uint32_t)(i * 512);
+                const float4 pa = lds128_u32(cur.addr + row_a + o), pb = lds128_u32(cur.addr + row_b + o);
+                const float4 xx = lds128_u32(x_u + (uint32_t)(q * INNER4 * 16) + o);
+                acc_a += (xlog2(xx.x, pa.x) + xlog2(xx.y, pa.y)) + (xlog2(xx.z, pa.z) + xlog2(xx.w, pa.w));
+                acc_b += (xlog2(xx.x, pb.x) + xlog2(xx.y, pb.y)) + (xlog2(xx.z, pb.z) + xlog2(xx.w, pb.w));
+                rsum_a += (pa.x + pa.y) + (pa.z + pa.w);
+                rsum_b += (pb.x + pb.y) + (pb.z + pb.w);
+            }
+        }
+        if (release) {  // forward only: the box is dead after its first read
+            __syncwarp();
+            if (lane == 0) mbar_arrive_u32(empty_u + cur.slot * 8);
+        }
+        cur.addr += slot_bytes;
+        if (++cur.slot == nslot) { cur.slot = 0; cur.addr = slots_u; cur.parity ^= 1u; }
+    }
+}
+
+// drate = g (x / r - 1) = (g x) rcp(r) - g
+__device__ __forceinline__ float4 drate4(const float4& r, const float4& xx, float g) {
+    return make_float4(fmaf(g * xx.x, fast_rcp(r.x), -g), fmaf(g * xx.y, fast_rcp(r.y), -g),
+                       fmaf(g * xx.z, fast_rcp(r.z), -g), fmaf(g * xx.w, fast_rcp(r.w), -g));
+}
+
+template <int INNER4, int NBOX>
+__device__ __forceinline__ void boxf_phase_b_poisson(uint32_t bs, uint32_t bs_addr, uint32_t slots_u, uint32_t slot_bytes,
+                                                     uint32_t nslot, uint32_t empty_u, uint32_t row_a, uint32_t row_b,
+                                                     uint32_t x_u, int lane, float ga, float gb, float* __restrict__ da,
+                                                     float* __restrict__ db, bool has_b) {
+    constexpr int VIT = (INNER4 + 31) / 32;
+#pragma unroll
+    for (int q = 0; q < NBOX; ++q) {
+#pragma unroll
+        for (int i = 0; i < VIT; ++i) {
+            if ((i + 1) * 32 <= INNER4 || lane + 32 * i < INNER4) {
+                const uint32_t o = (uint32_t)(i * 512);
+                const float4 pa = lds128_u32(bs_addr + row_a + o), pb = lds128_u32(bs_addr + row_b + o);
+                const float4 xx = lds128_u32(x_u + (uint32_t)(q * INNER4 * 16) + o);
+                stg_hint(da + q * INNER4 * 4 + i * 128, drate4(pa, xx, ga), 0);
+                if (has_b) stg_hint(db + q * INNER4 * 4 + i * 128, drate4(pb, xx, gb), 0);
+            }
+        }
+        __syncwarp();
+        if (lane == 0) mbar_arrive_u32(empty_u + bs * 8);
+        bs_addr += slot_bytes;
+        if (++bs == nslot) { bs = 0; bs_addr = slots_u; }
+    }
+}
+
 template <int EST, int INNER4, int NBOX, bool LOGITS>
 __global__ void __launch_bounds__((BOX_MAX_ROW_WARPS + 4) * 32, 1)
     k_iw_bernoulli_boxf(const __grid_constant__ CUtensorMap probs_map, float* __restrict__ cost,
@@ -1285,6 +1379,166 @@ __global__ void __launch_bounds__((BOX_MAX_ROW_WARPS + 4) * 32, 1)
     }
 }
 
+// Poisson likelihood over rates [K,B,X] (zs_iw_poisson_fused): the roles, barriers, staging pipeline and objective of
+// k_iw_bernoulli_boxf with the Poisson stager and row loops above; `probs_map` maps the rates, `dprobs` receives drate.
+// A kernel of its own rather than a likelihood parameter of k_iw_bernoulli_boxf: routing both through one inlined body
+// changed the register allocation of the Bernoulli instantiations, which stay as they were.
+template <int EST, int INNER4, int NBOX>
+__global__ void __launch_bounds__((BOX_MAX_ROW_WARPS + 4) * 32, 1)
+    k_iw_poisson_boxf(const __grid_constant__ CUtensorMap probs_map, float* __restrict__ cost,
+                      float* __restrict__ dprobs, float* __restrict__ dlogp, float* __restrict__ dlogq,
+                      float* __restrict__ logpx_out, const float* __restrict__ x,
+                      const float* __restrict__ logp_other, const float* __restrict__ logq, int K, int64_t B,
+                      int nslot, float gscale, int stagger_groups, int stagger_cycles, int flags, int64_t ldkb,
+                      float* __restrict__ loss_out, unsigned* __restrict__ ticket) {
+    extern __shared__ __align__(128) unsigned char smem[];
+    constexpr int INNER = INNER4 * 4, X = INNER * NBOX, X4 = X / 4;
+    const BoxLayout L(K, X, INNER, nslot);
+    const int Kpad = L.Kpad;
+    const uint32_t slot_bytes = (uint32_t)L.slot_bytes();
+    unsigned char* slots = smem + L.slots_off();
+    float* s_x = reinterpret_cast<float*>(smem + L.x_off());
+    double* s_xw = reinterpret_cast<double*>(smem + L.xw_off());
+    double* s_xv = reinterpret_cast<double*>(smem + L.xv_off());
+    float* s_lpx = reinterpret_cast<float*>(smem + L.lpx_off());
+    float* s_other = reinterpret_cast<float*>(smem + L.other_off());
+    float* s_lq = reinterpret_cast<float*>(smem + L.lq_off());
+    int* s_bin = reinterpret_cast<int*>(smem + L.bin_off());
+    uint64_t* full = reinterpret_cast<uint64_t*>(smem + L.bar_off());
+    uint64_t* empty = full + nslot;
+
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    // warp roles: [0, NW) row warps | NW stager | NW+1, NW+2 objective warps (even / odd columns) | NW+3 producer
+    const int NW = (blockDim.x >> 5) - 4;
+    const uint32_t box_bytes = (uint32_t)K * (uint32_t)INNER * 4u;
+    const float LN2 = 0.6931471805599453f;
+    const int64_t ncols = ((int64_t)blockIdx.x < B) ? (B - blockIdx.x + gridDim.x - 1) / gridDim.x : 0;
+
+    if (threadIdx.x == 0) {
+        for (int s = 0; s < nslot; ++s) {
+            mbar_init(&full[s], 1);
+            mbar_init(&empty[s], (uint32_t)NW);
+        }
+        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    }
+    auto stage_scalars = [&](int64_t b, int buf) { stage_scalars_batched(s_other + buf * Kpad, s_lq + buf * Kpad, logp_other, logq, K, ldkb, b, lane); };
+    // s_bin[slot] holds the bits of the column's C_b (the Bernoulli kernel keeps its binary-x flag there)
+    auto stage_x = [&](int64_t b, int slot) { stage_x_poisson(s_x + (size_t)slot * 2 * X, s_bin + slot, x + b * X, X4, lane); };
+    const bool is_stager = warp == NW, is_obj = warp == NW + 1 || warp == NW + 2, is_producer = warp == NW + 3;
+    pdl_wait();  // everything above touched shared memory only; probs / x / the [K,B] terms may come from the kernel before
+    pdl_trigger();
+    stagger_start(stagger_groups, stagger_cycles);
+    // Column 0 only: column 1 is staged while column 0 is being read.  The first tensor copies are issued AFTER
+    // this staging on purpose: issuing them first (measured here and in the ring kernel: +4 and +7 us per launch)
+    // starts every CTA's column 0 at the same instant, and the chip then alternates between a read-only phase A
+    // and a write-heavy phase B in lock-step; the variable staging latency spreads the CTAs out.
+    if (is_stager && ncols > 0) {
+        stage_scalars(blockIdx.x, 0);
+        stage_x(blockIdx.x, 0);
+    }
+    __syncthreads();
+
+    if (is_producer) {
+        // box t = (column t / NBOX, piece t % NBOX) goes to slot t % nslot
+        if (lane == 0) {
+            int slot = 0, q = 0;
+            uint32_t wait_parity = 1;
+            bool first_pass = true;
+            int64_t col = blockIdx.x;
+            const int64_t ntask = ncols * NBOX;
+            for (int64_t t = 0; t < ntask; ++t) {
+                if (!first_pass) mbar_wait(&empty[slot], wait_parity);
+                mbar_expect_tx(&full[slot], box_bytes);
+                tma_load_box(slots + (size_t)slot * slot_bytes, &probs_map, q * INNER, (int)col, 0, &full[slot]);
+                if (++q == NBOX) { q = 0; col += gridDim.x; }
+                if (++slot == nslot) {
+                    slot = 0;
+                    if (first_pass) { first_pass = false; wait_parity = 0; }
+                    else wait_parity ^= 1u;
+                }
+            }
+        }
+        return;
+    }
+    const int sync_threads = (NW + 2) * 32;
+    if (is_stager) {
+        int64_t b = blockIdx.x;
+        if (ncols > 1) {
+            stage_scalars(b + gridDim.x, 1);
+            stage_x(b + gridDim.x, 1);
+        }
+        for (int64_t c = 0; c < ncols; ++c, b += gridDim.x) {
+            named_bar_sync(1 + (int)(c & 1), sync_threads);
+            if (c + 2 < ncols) {
+                stage_scalars(b + 2 * (int64_t)gridDim.x, (int)((c + 2) & 3));
+                stage_x(b + 2 * (int64_t)gridDim.x, (int)((c + 2) % 3));
+            }
+        }
+        return;
+    }
+    if (is_obj) {
+        const int p = warp - NW - 1;
+        int64_t b = (int64_t)blockIdx.x + (int64_t)p * gridDim.x;
+        double part = 0.0;
+        for (int64_t c = p; c < ncols; c += 2, b += 2 * (int64_t)gridDim.x) {
+            const int buf = (int)(c & 3);
+            named_bar_sync(1 + p, sync_threads);
+            part += (double)column_objective<EST>(lane, K, ldkb, b, s_lpx + buf * Kpad, s_other + buf * Kpad,
+                                                  s_lq + buf * Kpad, s_xw + p * Kpad, gscale, cost, dlogp, dlogq,
+                                                  logpx_out, flags);
+        }
+        finish_loss(lane, p, part, loss_out, ticket);
+        return;
+    }
+
+    // ---- row warps: rows ka = warp and kb = warp + NW of every column (kb may not exist) ----------------
+    const int ka = warp, kb = warp + NW;
+    const bool has_b = kb < K;
+    const int kb_eff = has_b ? kb : ka;
+    const uint32_t slots_u = smem_u32(slots), full_u = smem_u32(full), empty_u = smem_u32(empty);
+    const uint32_t row_a = (uint32_t)ka * (INNER * 4) + (uint32_t)lane * 16, row_b = (uint32_t)kb_eff * (INNER * 4) + (uint32_t)lane * 16;
+    const uint32_t sx_u = smem_u32(s_x) + (uint32_t)lane * 16;
+    BoxCursor cur{0u, slots_u, 0u};
+    int64_t b = blockIdx.x;
+    for (int64_t c = 0; c < ncols; ++c, b += gridDim.x) {
+        const int par = (int)(c & 3), xs = (int)(c % 3);
+        const uint32_t x_u = sx_u + (uint32_t)xs * (2 * X * 4);
+        // the stager publishes column 1's x only after the first rendezvous of column 0 for c >= 2; column 1's
+        // staging is ordered by the rendezvous of column 0 as well (the stager arrives after staging it)
+        const uint32_t slot0 = cur.slot, addr0 = cur.addr;
+        const float cb = __int_as_float(s_bin[xs]);
+        float acc_a = 0.f, acc_b = 0.f, rsum_a = 0.f, rsum_b = 0.f;
+        boxf_phase_a_poisson<INNER4, NBOX>(cur, slots_u, slot_bytes, (uint32_t)nslot, full_u, empty_u, row_a, row_b,
+                                           x_u, lane, dprobs == nullptr, acc_a, acc_b, rsum_a, rsum_b);
+        acc_a = warp_sum(acc_a);
+        acc_b = warp_sum(acc_b);
+        rsum_a = warp_sum(rsum_a);
+        rsum_b = warp_sum(rsum_b);
+        if (lane == 0) {
+            const float la = (acc_a * LN2 - rsum_a) - cb;
+            s_lpx[par * Kpad + ka] = la;
+            s_xv[par * Kpad + ka] = ((double)la - (double)s_lq[par * Kpad + ka]) + (double)s_other[par * Kpad + ka];
+            if (has_b) {
+                const float lb = (acc_b * LN2 - rsum_b) - cb;
+                s_lpx[par * Kpad + kb] = lb;
+                s_xv[par * Kpad + kb] = ((double)lb - (double)s_lq[par * Kpad + kb]) + (double)s_other[par * Kpad + kb];
+            }
+        }
+        named_bar_sync(1 + (int)(c & 1), sync_threads);
+        if (dprobs) {
+            double m1;
+            float invS;
+            ring_max_sumexp(lane, K, s_xv + par * Kpad, m1, invS);
+            const float ga = -(expf((float)(s_xv[par * Kpad + ka] - m1)) * invS) * gscale;
+            const float gb = -(expf((float)(s_xv[par * Kpad + kb_eff] - m1)) * invS) * gscale;
+            float* da = dprobs + ((int64_t)ka * B + b) * X + lane * 4;
+            float* db = dprobs + ((int64_t)kb_eff * B + b) * X + lane * 4;
+            boxf_phase_b_poisson<INNER4, NBOX>(slot0, addr0, slots_u, slot_bytes, (uint32_t)nslot, empty_u, row_a,
+                                               row_b, x_u, lane, ga, gb, da, db, has_b);
+        }
+    }
+}
+
 static int pick_warps_ring(int K) {
     // row warps (three more warps stage inputs and compute the objective); equal rows per warp if possible
     for (int d = ZS_RING_MAX_ROW_WARPS; d >= 4; --d)
@@ -1348,6 +1602,7 @@ struct FusedCall {
     cudaStream_t st;
     float* loss_out = nullptr;   // sum_b cost[b], written by the launch itself (finish_loss), or null
     unsigned* ticket = nullptr;  // its workspace: counter word + per-warp partial sums (finish_loss)
+    bool poisson = false;        // `probs` holds Poisson rates, `x` counts (zs_iw_poisson_fused)
 };
 
 // Tensor map of probs[K][B][X] with box {inner, 1, K}; the driver's encoder is looked up through the runtime.
@@ -1461,8 +1716,9 @@ int launch_fused_box(const FusedCall& c, bool generic_only) {
         const bool sg = c.estimator == ZS_EST_SGVB;
 #define ZS_BOXF_PICK(I4, NB)                                                                                        \
     if (inner == 4 * (I4) && nbox == (NB))                                                                           \
-        fixed = c.logits ? (sg ? k_iw_bernoulli_boxf<ZS_EST_SGVB, I4, NB, true> : k_iw_bernoulli_boxf<ZS_EST_VIMCO, I4, NB, true>) \
-                         : (sg ? k_iw_bernoulli_boxf<ZS_EST_SGVB, I4, NB, false> : k_iw_bernoulli_boxf<ZS_EST_VIMCO, I4, NB, false>)
+        fixed = c.poisson ? (sg ? k_iw_poisson_boxf<ZS_EST_SGVB, I4, NB> : k_iw_poisson_boxf<ZS_EST_VIMCO, I4, NB>)      \
+              : c.logits  ? (sg ? k_iw_bernoulli_boxf<ZS_EST_SGVB, I4, NB, true> : k_iw_bernoulli_boxf<ZS_EST_VIMCO, I4, NB, true>) \
+                          : (sg ? k_iw_bernoulli_boxf<ZS_EST_SGVB, I4, NB, false> : k_iw_bernoulli_boxf<ZS_EST_VIMCO, I4, NB, false>)
         ZS_BOXF_PICK(28, 7);   // X = 784
         ZS_BOXF_PICK(32, 1);   // X = 128
         ZS_BOXF_PICK(64, 1);   // X = 256
@@ -1475,11 +1731,12 @@ int launch_fused_box(const FusedCall& c, bool generic_only) {
         launch_pdl(PDL_FUSED, fixed, dim3((unsigned)grid), dim3(threads), smem, c.st, map, c.cost, c.dprobs, c.dlogp, c.dlogq,
                    c.logpx_out, c.x, c.logp_other, c.logq, (int)K, B, nslot, (float)c.grad_scale, stg.groups, stg.cycles,
                    c.kflags, c.ldkb, c.loss_out, c.ticket);
-        ZS_LAUNCH_CHECK("k_iw_bernoulli_boxf");
+        ZS_LAUNCH_CHECK(c.poisson ? "k_iw_poisson_boxf" : "k_iw_bernoulli_boxf");
         return ZS_OK;
     }
-    if (c.logits) {
-        set_last_error_msg("fused logits form: no fixed-geometry kernel instantiated for this row length");
+    if (c.logits || c.poisson) {
+        set_last_error_msg(c.poisson ? "fused Poisson step: no fixed-geometry kernel instantiated for this row length"
+                                     : "fused logits form: no fixed-geometry kernel instantiated for this row length");
         return ZS_ERR_UNSUPPORTED;
     }
     auto kern = c.estimator == ZS_EST_SGVB ? k_iw_bernoulli_box<ZS_EST_SGVB> : k_iw_bernoulli_box<ZS_EST_VIMCO>;
@@ -1495,8 +1752,8 @@ int launch_fused_box(const FusedCall& c, bool generic_only) {
 
 int launch_fused_ring(const FusedCall& c) {
     const int64_t K = c.K, B = c.B, X = c.X;
-    if (c.logits) {
-        set_last_error_msg("fused logits form: only the fixed-geometry box kernels take logits");
+    if (c.logits || c.poisson) {
+        set_last_error_msg("fused logits / Poisson form: only the fixed-geometry box kernels take it");
         return ZS_ERR_UNSUPPORTED;
     }
     int max_optin = 0;
@@ -1592,6 +1849,41 @@ int zs_iw_bernoulli_fused_loss(int estimator, float* loss_out, void* workspace, 
     ZS_REQUIRE(persistent_grid(B) <= ZS_FUSED_LOSS_MAX_GRID, ZS_ERR_UNSUPPORTED);
     c.loss_out = loss_out;
     c.ticket = (unsigned*)workspace;
+    return fused_launch(c);
+}
+
+int zs_iw_poisson_fused(int estimator, float* cost, float* drate, float* dlogp, float* dlogq, float* logpx_out,
+                        const float* rate, const float* x, const float* logp_other, const float* logq, int64_t K,
+                        int64_t B, int64_t X, double grad_scale, int flags, zs_stream_t stream) {
+    ZS_REQUIRE(rate && x && K >= 1 && B >= 0 && X >= 1, ZS_ERR_ARG);
+    ZS_REQUIRE(estimator == ZS_EST_SGVB || estimator == ZS_EST_VIMCO, ZS_ERR_ARG);
+    ZS_REQUIRE(!(estimator == ZS_EST_VIMCO && (K < 2 || logq == nullptr)), ZS_ERR_ARG);
+    ZS_REQUIRE((flags & ~(ZS_FUSED_ACCUMULATE_COST | ZS_FUSED_COST_SCALED)) == 0, ZS_ERR_ARG);
+    if (B == 0) return ZS_OK;
+    FusedCall c{estimator, cost, drate, dlogp, dlogq, logpx_out, rate, x, logp_other, logq, K, B, X, B, grad_scale,
+                ((flags & ZS_FUSED_ACCUMULATE_COST) ? FUSED_ACCUMULATE : 0) |
+                    ((flags & ZS_FUSED_COST_SCALED) ? FUSED_COST_SCALED : 0),
+                false, as_stream(stream)};
+    c.poisson = true;
+    return fused_launch(c);
+}
+
+int zs_iw_poisson_fused_loss(int estimator, float* loss_out, void* workspace, float* cost, float* drate, float* dlogp,
+                             float* dlogq, float* logpx_out, const float* rate, const float* x, const float* logp_other,
+                             const float* logq, int64_t K, int64_t B, int64_t X, double grad_scale, int flags,
+                             zs_stream_t stream) {
+    ZS_REQUIRE(rate && x && loss_out && workspace && cost && K >= 1 && B >= 1 && X >= 1, ZS_ERR_ARG);
+    ZS_REQUIRE(estimator == ZS_EST_SGVB || estimator == ZS_EST_VIMCO, ZS_ERR_ARG);
+    ZS_REQUIRE(!(estimator == ZS_EST_VIMCO && (K < 2 || logq == nullptr)), ZS_ERR_ARG);
+    ZS_REQUIRE((flags & ~(ZS_FUSED_ACCUMULATE_COST | ZS_FUSED_COST_SCALED)) == 0, ZS_ERR_ARG);
+    FusedCall c{estimator, cost, drate, dlogp, dlogq, logpx_out, rate, x, logp_other, logq, K, B, X, B, grad_scale,
+                ((flags & ZS_FUSED_ACCUMULATE_COST) ? FUSED_ACCUMULATE : 0) |
+                    ((flags & ZS_FUSED_COST_SCALED) ? FUSED_COST_SCALED : 0),
+                false, as_stream(stream)};
+    ZS_REQUIRE(persistent_grid(B) <= ZS_FUSED_LOSS_MAX_GRID, ZS_ERR_UNSUPPORTED);
+    c.loss_out = loss_out;
+    c.ticket = (unsigned*)workspace;
+    c.poisson = true;
     return fused_launch(c);
 }
 

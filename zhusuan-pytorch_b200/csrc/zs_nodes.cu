@@ -1,4 +1,4 @@
-// Stochastic-node kernels: sample and log-prob (forward / backward) for Normal and Bernoulli
+// Stochastic-node kernels: sample and log-prob (forward / backward) for Normal, Bernoulli and Poisson
 // over the [K, M, E] particle-row view described in include/zs_b200.h.
 //
 // Replaces (reference file:line):
@@ -193,6 +193,28 @@ struct BernoulliLogitsOp<double> {
         double dp;
         BernoulliOp<double>::grad<NEED_X>(g, x, p, 0.0, dx, dp, unused);
         dl = dp * ((1.0 - p) * p);
+    }
+};
+
+__device__ __forceinline__ float lgamma_t(float v) { return lgammaf(v); }
+__device__ __forceinline__ double lgamma_t(double v) { return ::lgamma(v); }
+
+// Poisson(rate): torch.distributions.Poisson.log_prob, which the reference's Poisson._log_prob calls
+// (zhusuan/distributions/poisson.py:75):  xlogy(x, rate) - rate - lgamma(x + 1).
+// xlogy is 0 at x == 0 unless rate is NaN, so rate == 0 gives 0 at x == 0 and -inf at x > 0.
+// d/drate = g (x / rate - 1), torch's xlogy backward; the count carries no gradient (the host refuses one).
+template <typename T>
+struct PoissonOp {
+    static __device__ __forceinline__ T term(T x, T rate, T) {
+        const T xl = (x == T(0) && !isnan(rate)) ? T(0) : x * Real<T>::log(rate);
+        return (xl - rate) - lgamma_t(x + T(1));
+    }
+    static __device__ __forceinline__ T finish(T acc) { return acc; }
+    template <bool NEED_X>
+    static __device__ __forceinline__ void grad(T g, T x, T rate, T, T& dx, T& drate, T& unused) {
+        drate = g * (x / rate - T(1));
+        dx = T(0);
+        unused = T(0);
     }
 };
 
@@ -714,6 +736,73 @@ __global__ void __launch_bounds__(256) k_bernoulli_sample(T* __restrict__ out, c
     }
 }
 
+// Poisson(rate) counts (torch.distributions.Poisson.sample as the reference calls it, zhusuan/distributions/poisson.py:61),
+// drawn as ATen's CPU sample_poisson does: Knuth's product of uniforms for rate < 10, Hormann's transformed rejection
+// (PTRS, "The transformed rejection method for generating Poisson random variables", 1993) for rate >= 10, in double
+// for both dtypes.  Element i reads its uniforms in order from the words of Philox groups j = 0, 1, ... at counter
+// i | (j << 48): a pure function of (seed, offset, i), whatever the launch geometry, and disjoint from the counters of
+// the next stream position (offset + ZS_RNG_TICK).  Knuth takes one word per step, PTRS two (U, V) per trial.
+// The loop stops after POISSON_MAX_WORDS words (64 groups): Knuth then returns 256, PTRS floor(rate).  For rate < 10
+// Knuth needs more than 256 words only if the count exceeds 255, P < 1e-250; a PTRS trial is rejected with probability
+// below 0.13 for rate >= 10, so 128 rejections in a row have P < 1e-113.  Rates are not validated (no host
+// synchronisation): a negative or NaN rate gives 0, rate must be finite.
+constexpr int POISSON_MAX_WORDS = 256;
+
+struct PhiloxWords {
+    uint64_t i, offset, seed;
+    uint32_t w[4];
+    int used;  // words consumed so far
+    __device__ __forceinline__ double next() {
+        if ((used & 3) == 0) {
+            const Philox4 r = philox4x32_10(i | ((uint64_t)(used >> 2) << 48), offset, seed);
+            w[0] = r.x; w[1] = r.y; w[2] = r.z; w[3] = r.w;
+        }
+        return (double)u01_closed_open(w[used++ & 3]);  // [0, 1), 24 bits
+    }
+};
+
+__device__ double poisson_draw(double lam, PhiloxWords& u) {
+    if (lam >= 10.0) {
+        const double slam = ::sqrt(lam), loglam = ::log(lam);
+        const double b = 0.931 + 2.53 * slam;
+        const double a = -0.059 + 0.02483 * b;
+        const double invalpha = 1.1239 + 1.1328 / (b - 3.4);
+        const double vr = 0.9277 - 3.6224 / (b - 2.0);
+        while (u.used < POISSON_MAX_WORDS) {
+            const double U = u.next() - 0.5;
+            const double V = u.next();
+            const double us = 0.5 - ::fabs(U);
+            const double k = ::floor((2.0 * a / us + b) * U + lam + 0.43);
+            if (us >= 0.07 && V <= vr) return k;
+            if (k < 0.0 || (us < 0.013 && V > us)) continue;
+            if (::log(V) + ::log(invalpha) - ::log(a / (us * us) + b) <= -lam + k * loglam - ::lgamma(k + 1.0)) return k;
+        }
+        return ::floor(lam);
+    }
+    if (lam == 0.0) return 0.0;
+    const double enlam = ::exp(-lam);
+    double x = 0.0, prod = 1.0;
+    while (u.used < POISSON_MAX_WORDS) {
+        prod *= u.next();
+        if (!(prod > enlam)) return x;
+        x += 1.0;
+    }
+    return x;
+}
+
+template <typename T>
+__global__ void __launch_bounds__(256) k_poisson_sample(T* __restrict__ out, const T* __restrict__ rate, int rm,
+                                                        int64_t K, int64_t N, uint64_t seed, uint64_t offset,
+                                                        unsigned long long* rs) {
+    offset = rng_acquire(offset, rs, nullptr, true);
+    const int64_t total = K * N;
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (int64_t)gridDim.x * blockDim.x) {
+        const T rv = rm == ZS_FULL ? rate[i] : (rm == ZS_KBCAST ? rate[i % N] : rate[0]);
+        PhiloxWords u{(uint64_t)i, offset, seed, {0u, 0u, 0u, 0u}, 0};
+        out[i] = (T)poisson_draw((double)rv, u);
+    }
+}
+
 template <typename T>
 __global__ void __launch_bounds__(256) k_philox_fill(T* __restrict__ out, int64_t n, T mean, T std, int normal,
                                                      uint64_t seed, uint64_t offset, unsigned long long* rs) {
@@ -1143,6 +1232,44 @@ int zs_bernoulli_logits_logpmf_bwd(int dtype, void* dx, void* dlogits, const voi
                                                      Operand<T>{(const T*)x, x_mode},
                                                      Operand<T>{(const T*)logits, logits_mode},
                                                      Operand<T>{nullptr, ZS_SCALAR}, K, M, E, as_stream(stream));
+    })
+}
+
+/* ---- Poisson stochastic node ---------------------------------------------------------------------------- */
+int zs_poisson_sample(int dtype, void* out, const void* rate, int rate_mode, int64_t K, int64_t N, uint64_t seed,
+                      uint64_t offset, void* rng_state, zs_stream_t stream) {
+    ZS_REQUIRE(out && rate && K >= 0 && N >= 0 && valid_mode(rate_mode), ZS_ERR_ARG);
+    if (K * N == 0) return ZS_OK;
+    ZS_REQUIRE(K * N < ((int64_t)1 << 48), ZS_ERR_UNSUPPORTED);  // element index below the group bits of the counter
+    const int grid = grid_for(K * N, 256);
+    ZS_DTYPE_SWITCH(dtype, {
+        k_poisson_sample<T><<<grid, 256, 0, as_stream(stream)>>>((T*)out, (const T*)rate, rate_mode, K, N, seed, offset,
+                                                                 rs_ptr(rng_state));
+    })
+    ZS_LAUNCH_CHECK("k_poisson_sample");
+    return ZS_OK;
+}
+
+int zs_poisson_logpmf_fwd(int dtype, void* out, const void* x, int x_mode, const void* rate, int rate_mode, int64_t K,
+                          int64_t M, int64_t E, zs_stream_t stream) {
+    ZS_REQUIRE(out && x && rate && K >= 0 && M >= 0 && E >= 1, ZS_ERR_ARG);
+    ZS_REQUIRE(valid_mode(x_mode) && valid_mode(rate_mode), ZS_ERR_ARG);
+    ZS_DTYPE_SWITCH(dtype, {
+        return dispatch_rows_fwd<T, PoissonOp<T>>((T*)out, Operand<T>{(const T*)x, x_mode},
+                                                  Operand<T>{(const T*)rate, rate_mode},
+                                                  Operand<T>{nullptr, ZS_SCALAR}, K, M, E, as_stream(stream));
+    })
+}
+
+int zs_poisson_logpmf_bwd(int dtype, void* drate, const void* g, const void* x, int x_mode, const void* rate,
+                          int rate_mode, int64_t K, int64_t M, int64_t E, zs_stream_t stream) {
+    ZS_REQUIRE(g && x && rate && K >= 0 && M >= 0 && E >= 1, ZS_ERR_ARG);
+    ZS_REQUIRE(valid_mode(x_mode) && valid_mode(rate_mode), ZS_ERR_ARG);
+    if (!drate) return ZS_OK;
+    ZS_DTYPE_SWITCH(dtype, {
+        return dispatch_bwd<T, PoissonOp<T>>((T*)nullptr, (T*)drate, (T*)nullptr, (const T*)g,
+                                             Operand<T>{(const T*)x, x_mode}, Operand<T>{(const T*)rate, rate_mode},
+                                             Operand<T>{nullptr, ZS_SCALAR}, K, M, E, as_stream(stream));
     })
 }
 

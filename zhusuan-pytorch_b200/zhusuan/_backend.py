@@ -65,6 +65,11 @@ def _declare(lib):
         "zs_locscale_sample_bwd": (i32, [i32, i32, vp, i32, vp, i32, vp, vp, i64, i64, u64, u64, vp, vp]),
         "zs_locscale_logprob_fwd": (i32, [i32, i32, vp, vp, i32, vp, i32, vp, i32, i64, i64, i64, vp]),
         "zs_locscale_logprob_bwd": (i32, [i32, i32, vp, vp, vp, vp, vp, i32, vp, i32, vp, i32, i64, i64, i64, vp]),
+        "zs_poisson_sample": (i32, [i32, vp, vp, i32, i64, i64, u64, u64, vp, vp]),
+        "zs_poisson_logpmf_fwd": (i32, [i32, vp, vp, i32, vp, i32, i64, i64, i64, vp]),
+        "zs_poisson_logpmf_bwd": (i32, [i32, vp, vp, vp, i32, vp, i32, i64, i64, i64, vp]),
+        "zs_iw_poisson_fused": (i32, [i32, vp, vp, vp, vp, vp, vp, vp, vp, vp, i64, i64, i64, dbl, i32, vp]),
+        "zs_iw_poisson_fused_loss": (i32, [i32, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, i64, i64, i64, dbl, i32, vp]),
         "zs_bernoulli_logits_logpmf_fwd": (i32, [i32, vp, vp, i32, vp, i32, i64, i64, i64, vp]),
         "zs_bernoulli_logits_logpmf_bwd": (i32, [i32, vp, vp, vp, vp, i32, vp, i32, i64, i64, i64, vp]),
         "zs_categorical_sample": (i32, [i32, vp, vp, i32, vp, i64, i64, i64, u64, u64, vp, vp]),
@@ -368,6 +373,32 @@ def bernoulli_logpmf_bwd(g, x, xm, probs, pm, K, M, E, need_x, need_probs, logit
     return dx, dprobs
 
 
+# ----------------------------------------------------------------------------- Poisson
+def poisson_sample(rate, rm, K, N, seed=0, offset=0, rng_state=None):
+    dt, dev = rate.dtype, rate.device
+    _chk(dev, dt, rate=rate)
+    _chk_state(dev, rng_state=rng_state)
+    out = torch.empty((K, N), dtype=dt, device=dev)
+    _go("zs_poisson_sample", dev, dtype_code(dt), _ptr(out), _ptr(rate), rm, K, N, seed, offset, _ptr(rng_state))
+    return out
+
+
+def poisson_logpmf_fwd(x, xm, rate, rm, K, M, E):
+    dt, dev = rate.dtype, rate.device
+    _chk(dev, dt, x=x, rate=rate)
+    out = torch.empty((K, M), dtype=dt, device=dev)
+    _go("zs_poisson_logpmf_fwd", dev, dtype_code(dt), _ptr(out), _ptr(x), xm, _ptr(rate), rm, K, M, E)
+    return out
+
+
+def poisson_logpmf_bwd(g, x, xm, rate, rm, K, M, E):
+    dt, dev = rate.dtype, rate.device
+    _chk(dev, dt, g=g, x=x, rate=rate)
+    drate = torch.empty_like(rate)
+    _go("zs_poisson_logpmf_bwd", dev, dtype_code(dt), _ptr(drate), _ptr(g), _ptr(x), xm, _ptr(rate), rm, K, M, E)
+    return drate
+
+
 # ----------------------------------------------------------------------------- Logistic / Laplace
 FAM_LOGISTIC, FAM_LAPLACE, FAM_UNIFORM = 1, 2, 3
 
@@ -502,6 +533,11 @@ def fused_logits_supported(K, X, dtype):
     return (nbox + 1) * (slot + 16) + fixed <= 227 * 1024
 
 
+def fused_poisson_supported(K, X, dtype):
+    """Shapes zs_iw_poisson_fused takes: the fixed-geometry box kernel, as for the logits form."""
+    return fused_logits_supported(K, X, dtype)
+
+
 def set_latent_fwd_impl(impl):
     """Developer hook: -1 = by shape, 0 = lane-per-unit forward, 1 = row-per-thread forward (zs_debug_set_latent_fwd)."""
     check(load().zs_debug_set_latent_fwd(int(impl)), "zs_debug_set_latent_fwd")
@@ -544,6 +580,21 @@ def iw_bernoulli_fused(estimator, probs, x, logp_other, logq, grad_scale, need_d
     grad_scale, so cost.sum() is the mean objective (ZS_FUSED_COST_SCALED).  `want_loss=True`: the launch also writes
     sum_b cost[b] into "loss" [1] (zs_iw_bernoulli_fused_loss); "loss" is None when no counter word is available.
     Returns dict(cost[B], dprobs, dlogp, dlogq, logpx, loss) or None when the shape is not supported."""
+    return _iw_fused("bernoulli", estimator, probs, x, logp_other, logq, grad_scale, need_dprobs, want_logpx, out,
+                     logits, accumulate_cost, cost_scaled, want_loss)
+
+
+def iw_poisson_fused(estimator, rate, x, logp_other, logq, grad_scale, need_drate=True, want_logpx=False, out=None,
+                     accumulate_cost=False, cost_scaled=False, want_loss=False):
+    """The fused step for a Poisson likelihood (zs_iw_poisson_fused[_loss]): rate [K,B,X], counts x [B,X]; the same
+    options and results as iw_bernoulli_fused, the gradient w.r.t. the rates under the key "dprobs".  None when the
+    shape is not supported."""
+    return _iw_fused("poisson", estimator, rate, x, logp_other, logq, grad_scale, need_drate, want_logpx, out, False,
+                     accumulate_cost, cost_scaled, want_loss)
+
+
+def _iw_fused(lik, estimator, probs, x, logp_other, logq, grad_scale, need_dprobs, want_logpx, out, logits,
+              accumulate_cost, cost_scaled, want_loss):
     dev = probs.device
     _chk(dev, torch.float32, probs=probs, x=x, logp_other=logp_other, logq=logq)
     K, B, X = probs.shape
@@ -561,11 +612,11 @@ def iw_bernoulli_fused(estimator, probs, x, logp_other, logq, grad_scale, need_d
     if ticket is not None:
         loss = o.get("loss") if "loss" in o else torch.empty(1, dtype=torch.float32, device=dev)
         _chk(dev, torch.float32, loss=loss)
-        name = "zs_iw_bernoulli_fused_loss"
+        name = "zs_iw_%s_fused_loss" % lik
         rc = _run(name, dev, estimator, _ptr(loss), ticket, _ptr(cost), _ptr(dprobs), _ptr(dlp), _ptr(dlq), _ptr(lpx),
                   _ptr(probs), _ptr(x), _ptr(logp_other), _ptr(logq), K, B, X, float(grad_scale), flags)
     else:
-        name = "zs_iw_bernoulli_fused"
+        name = "zs_iw_%s_fused" % lik
         rc = _run(name, dev, estimator, _ptr(cost), _ptr(dprobs), _ptr(dlp), _ptr(dlq), _ptr(lpx),
                   _ptr(probs), _ptr(x), _ptr(logp_other), _ptr(logq), K, B, X, float(grad_scale), flags)
     if rc in (ERR_UNSUPPORTED, ERR_ALIGN):

@@ -649,6 +649,64 @@ def bernoulli_sample(probs, n_samples):
 
 
 # --------------------------------------------------------------------------------------------
+# Poisson
+# --------------------------------------------------------------------------------------------
+class _PoissonLogPmf(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, x, rate, modes, K, M, E):
+        out = be.poisson_logpmf_fwd(x, modes[0], rate, modes[1], K, M, E)
+        ctx.save_for_backward(x, rate)
+        ctx.cfg = (modes, K, M, E)
+        return out
+
+    @staticmethod
+    def backward(ctx, g):
+        x, rate = ctx.saved_tensors
+        modes, K, M, E = ctx.cfg
+        drate = be.poisson_logpmf_bwd(g.contiguous(), x, modes[0], rate, modes[1], K, M, E) if ctx.needs_input_grad[1] \
+            else None
+        return None, drate, None, None, None, None
+
+
+def _no_count_grad(x):
+    if torch.is_tensor(x) and x.requires_grad:
+        raise ValueError("Poisson.log_prob: the counts have no gradient (the log-pmf is defined at integers); "
+                         "pass a tensor that does not require grad (e.g. x.detach())")
+
+
+def poisson_log_prob(x, rate, n_event):
+    """sum over the last n_event axes of xlogy(x, rate) - rate - lgamma(x + 1) (the reference's poisson.py:75,
+    torch.distributions.Poisson.log_prob); the gradient reaches `rate` only."""
+    _no_count_grad(x)
+    home = rate.device
+    x, rate = to_compute(x), to_compute(rate)
+    L = Layout([x.shape, rate.shape], n_event)
+    if _prod(L.S) == 0:
+        return back_home(torch.zeros(L.lead, dtype=rate.dtype, device=rate.device), home)
+    (xc, xm), (rc, rm) = L.canon(x), L.canon(rate)
+    if rm == SCALAR:  # as for Bernoulli: a gradient w.r.t. a SCALAR operand is the host's job, so expand it
+        rc, rm = rate.expand(L.S).contiguous(), FULL
+    out = _PoissonLogPmf.apply(xc, rc, (xm, rm), L.K, L.M, L.E)
+    return back_home(out.reshape(L.lead), home)
+
+
+def poisson_sample(rate, n_samples):
+    """Poisson._sample (the reference's poisson.py:61): float counts, [n_samples] + rate.shape (no leading axis
+    for n_samples 1), drawn in-kernel from Philox uniforms; no gradient."""
+    home = rate.device
+    rate = to_compute(rate).detach()
+    K = int(n_samples)
+    base = tuple(rate.shape)
+    out_shape = ((K,) if K > 1 else ()) + base
+    N = _prod(base)
+    if N == 0:
+        return back_home(torch.zeros(out_shape, dtype=rate.dtype, device=rate.device), home)
+    kw, _ = _draw_kwargs(rate.device, None)
+    out = be.poisson_sample(rate.contiguous(), KBCAST if K > 1 else FULL, K, N, **kw)
+    return back_home(out.reshape(out_shape), home)
+
+
+# --------------------------------------------------------------------------------------------
 # Categorical (not in the reference; see distributions/categorical.py)
 # --------------------------------------------------------------------------------------------
 class _CategoricalLogPmf(torch.autograd.Function):
@@ -880,6 +938,35 @@ def iw_bernoulli_fused(probs, x, logp_other, logq, estimator, logits=False):
     lo = None if logp_other is None else logp_other.contiguous()
     lq = None if logq is None else logq.contiguous()
     return _IWBernoulliFused.apply(probs, x, lo, lq, estimator, bool(logits))
+
+
+class _IWPoissonFused(torch.autograd.Function):
+    """Poisson likelihood + IW objective, forward and backward in ONE launch (zs_iw_poisson_fused_loss); the
+    upstream scalar is applied in backward exactly as for _IWBernoulliFused."""
+
+    @staticmethod
+    def forward(ctx, rate, x, logp_other, logq, estimator):
+        K, B, X = rate.shape
+        r = be.iw_poisson_fused(estimator, rate, x, logp_other, logq, _mean_scale(B), need_drate=ctx.needs_input_grad[0],
+                                cost_scaled=True, want_loss=True)
+        if r is None:
+            raise be.BackendError("fused Poisson IW kernel refused a shape fused_poisson_supported() accepted")
+        ctx.grads = (r["dprobs"], r["dlogp"], r["dlogq"])
+        loss = r.get("loss")
+        return loss.reshape(()) if loss is not None else r["cost"].sum()
+
+    @staticmethod
+    def backward(ctx, g):
+        return _IWBernoulliFused.backward(ctx, g)[:5]  # same gradient buffers; one input (`logits`) fewer
+
+
+def iw_poisson_fused(rate, x, logp_other, logq, estimator):
+    """rate [K,B,X] (CUDA, float32), counts x [B,X], logp_other / logq [K,B] or None -> scalar loss."""
+    rate = _aligned(rate)
+    x = _aligned(x.to(rate.dtype))
+    lo = None if logp_other is None else logp_other.contiguous()
+    lq = None if logq is None else logq.contiguous()
+    return _IWPoissonFused.apply(rate, x, lo, lq, estimator)
 
 
 # --------------------------------------------------------------------------------------------

@@ -2,15 +2,15 @@
 
 Same attributes (`_nodes`, `_cache`, `_observed`, `_device`), properties and methods as the
 reference (:72-240): `observe`, `stochastic_node` / `sn` / `snode`, the per-distribution aliases of
-the hot-path distributions, `log_joint` / `_log_joint`.  Only Normal, Bernoulli and Categorical are
-registered: the other aliases of the reference (beta, gamma, ...) wrap torch.distributions and are
-outside the accelerated path.
+the hot-path distributions, `log_joint` / `_log_joint`.  Normal, Bernoulli, Categorical, Logistic, Laplace,
+Uniform and Poisson are registered: the other aliases of the reference (beta, gamma, ...) wrap
+torch.distributions and are outside the accelerated path.
 """
 import torch
 import torch.nn as nn
 
 from zhusuan.framework.stochastic_tensor import StochasticTensor
-from zhusuan.distributions import Distribution, Normal, Bernoulli, Categorical, Logistic, Laplace, Uniform
+from zhusuan.distributions import Distribution, Normal, Bernoulli, Categorical, Logistic, Laplace, Uniform, Poisson
 
 __all__ = ['BayesianNet']
 
@@ -21,9 +21,10 @@ name_mapping = {
     "Logistic": Logistic,
     "Laplace": Laplace,
     "Uniform": Uniform,
+    "Poisson": Poisson,
 }
 
-_OUT_OF_SCOPE = ("Beta", "Exponential", "Gamma", "Poisson", "StudentT")
+_OUT_OF_SCOPE = ("Beta", "Exponential", "Gamma", "StudentT")
 
 
 class BayesianNet(nn.Module):
@@ -116,6 +117,13 @@ class BayesianNet(nn.Module):
             raise ValueError("name of stochastic_node must be str")
         dist = Categorical(logits=logits, probs=probs, dtype=dtype, is_continuous=is_continuous,
                            group_ndims=group_ndims, device=self.device, **kwargs)
+        return self._register(name, dist, n_samples, kwargs)
+
+    def poisson(self, name, rate, dtype=None, is_continuous=False, group_ndims=0, n_samples=None, **kwargs):
+        if not isinstance(name, str):
+            raise ValueError("name of stochastic_node must be str")
+        dist = Poisson(rate=rate, dtype=dtype, is_continuous=is_continuous, group_ndims=group_ndims,
+                       device=self.device, **kwargs)
         return self._register(name, dist, n_samples, kwargs)
 
     def laplace(self, name, loc, scale, dtype=None, is_continuous=True, group_ndims=0, n_samples=None, **kwargs):

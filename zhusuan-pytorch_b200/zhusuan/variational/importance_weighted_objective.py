@@ -5,7 +5,8 @@ Both estimators run as ONE kernel over the [K,B] log-weights that produces the s
 its gradient (the reference launches ~40 aten kernels and, for VIMCO, materialises a [B,K,K] tensor,
 :164-191).  When the generator's likelihood is a Bernoulli node over [K,B,X] probabilities, the
 likelihood log-pmf, the objective and the likelihood's backward are fused further into the
-resident-column kernel (zs_iw_bernoulli_fused): probs is read from HBM once, dprobs written once.
+resident-column kernel (zs_iw_bernoulli_fused): probs is read from HBM once, dprobs written once.  A Poisson
+likelihood over [K,B,X] rates takes the same kernel's Poisson form (zs_iw_poisson_fused).
 """
 import torch
 from zhusuan._shapes import broadcast_shapes as _bshapes
@@ -13,6 +14,7 @@ import torch.nn as nn
 
 from zhusuan.framework.stochastic_tensor import StochasticTensor
 from zhusuan.distributions.bernoulli import Bernoulli
+from zhusuan.distributions.poisson import Poisson
 from zhusuan import _ops
 from zhusuan import _backend as _be
 
@@ -57,17 +59,19 @@ class ImportanceWeightedObjective(nn.Module):
 
     # -- fused path -----------------------------------------------------------------------------
     def _fusable_likelihood(self, nodes_p):
-        """Name of a generator node that is an observed Bernoulli likelihood over [K,B,X] probabilities
-        whose only reduction is the sum over X — the shape the fused kernel handles — else None."""
+        """Name of a generator node that is an observed Bernoulli likelihood over [K,B,X] probabilities, or an observed
+        Poisson likelihood over device-resident [K,B,X] rates, whose only reduction is the sum over X — the shape the
+        fused kernel handles — else None."""
         from zhusuan import variational as _v
         if not _v.FUSED or self._axis != 0:
             return None
         best, best_numel = None, 0
         for name, node in nodes_p.items():
-            if not isinstance(node, StochasticTensor) or not isinstance(node.dist, Bernoulli):
+            if not isinstance(node, StochasticTensor) or not isinstance(node.dist, (Bernoulli, Poisson)):
                 continue
-            logits = node.dist.from_logits
-            probs = node.dist.probs if logits is None else logits  # the kernel's [K,B,X] operand
+            poisson = isinstance(node.dist, Poisson)
+            logits = None if poisson else node.dist.from_logits
+            probs = node.dist.rate if poisson else (node.dist.probs if logits is None else logits)  # [K,B,X] operand
             x = node._observed_value()
             if x is None or not torch.is_tensor(x) or probs.dim() != 3:
                 continue
@@ -78,7 +82,12 @@ class ImportanceWeightedObjective(nn.Module):
             n_event, mean_dims, sum_dims = node.reduction_plan(x.shape)
             if n_event != 1 or mean_dims or sum_dims:
                 continue
-            if logits is not None:
+            if poisson:
+                # device-resident rates only (host-resident ones take the generic path), instantiated row lengths
+                if not _be.on_compute_device(probs) or not _be.fused_poisson_supported(
+                        int(probs.shape[0]), int(probs.shape[2]), probs.dtype):
+                    continue
+            elif logits is not None:
                 # the logits form exists on the device-resident route, for the instantiated row lengths
                 if not _be.on_compute_device(probs) or not _be.fused_logits_supported(
                         int(probs.shape[0]), int(probs.shape[2]), probs.dtype):
@@ -91,8 +100,9 @@ class ImportanceWeightedObjective(nn.Module):
 
     def _forward_fused(self, nodes_p, nodes_q, lik):
         node = nodes_p[lik]
-        logits = node.dist.from_logits
-        probs = node.dist.probs if logits is None else logits
+        poisson = isinstance(node.dist, Poisson)
+        logits = None if poisson else node.dist.from_logits
+        probs = node.dist.rate if poisson else (node.dist.probs if logits is None else logits)
         K, B = int(probs.shape[0]), int(probs.shape[1])
         x = node._observed_value()
         node.dist.sample_cache = x
@@ -128,6 +138,8 @@ class ImportanceWeightedObjective(nn.Module):
             return _ops.iw_bernoulli_fused_host(probs, x.to(dev), logp_other, logq, est)
         lo = None if logp_other is None else logp_other.to(dev, probs.dtype)
         lq = None if logq is None else logq.to(dev, probs.dtype)
+        if poisson:
+            return _ops.iw_poisson_fused(probs, x.to(dev), lo, lq, est)
         return _ops.iw_bernoulli_fused(probs, x.to(dev), lo, lq, est, logits=logits is not None)
 
     # -- reference protocol ---------------------------------------------------------------------
