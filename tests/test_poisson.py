@@ -412,7 +412,7 @@ def test_fused_kernel_dispatch_and_fallback():
 @pytest.mark.parametrize("est", [_backend.SGVB, _backend.VIMCO])
 def test_fused_kernel_entry_point_against_restatement(est):
     """zs_iw_poisson_fused at each instantiated row length (K = 50 and K = 7), against the oracle restatement; with
-    counts that are mostly zero, and rates that reach 0 (log-weight -inf only where the count is positive)."""
+    counts that are mostly zero and rates of at least 0.01 (zero and subnormal rates: tests/test_fused_box_columns.py)."""
     import poisson_oracle
     rng = np.random.RandomState(24)
     for X, K in ((128, 50), (256, 7), (512, 50), (784, 50), (1024, 33)):

@@ -1150,7 +1150,20 @@ __device__ __forceinline__ void stage_x_poisson(float* s_xrow, int* s_cb, const 
     c = warp_sum(c);
     if (lane == 0) *s_cb = __float_as_int(c);
 }
-__device__ __forceinline__ float xlog2(float x, float r) { return x == 0.f ? 0.f : x * fast_log2(r); }
+// The Poisson row loops use the SFU's log2 and reciprocal WITHOUT flush-to-zero: a subnormal rate (exp(l) for a decoder
+// output l < -87.3) with a positive count has a finite x log r in torch and in the two-pass route's logf, where the
+// .ftz forms would read it as 0 and give -inf (a NaN column when every particle does so).
+__device__ __forceinline__ float log2_approx_sub(float x) {
+    float y;
+    asm("lg2.approx.f32 %0, %1;" : "=f"(y) : "f"(x));
+    return y;
+}
+__device__ __forceinline__ float rcp_approx_sub(float x) {
+    float y;
+    asm("rcp.approx.f32 %0, %1;" : "=f"(y) : "f"(x));
+    return y;
+}
+__device__ __forceinline__ float xlog2(float x, float r) { return x == 0.f ? 0.f : x * log2_approx_sub(r); }
 
 template <int INNER4, int NBOX>
 __device__ __forceinline__ void boxf_phase_a_poisson(BoxCursor& cur, uint32_t slots_u, uint32_t slot_bytes, uint32_t nslot,
@@ -1184,8 +1197,8 @@ __device__ __forceinline__ void boxf_phase_a_poisson(BoxCursor& cur, uint32_t sl
 
 // drate = g (x / r - 1) = (g x) rcp(r) - g
 __device__ __forceinline__ float4 drate4(const float4& r, const float4& xx, float g) {
-    return make_float4(fmaf(g * xx.x, fast_rcp(r.x), -g), fmaf(g * xx.y, fast_rcp(r.y), -g),
-                       fmaf(g * xx.z, fast_rcp(r.z), -g), fmaf(g * xx.w, fast_rcp(r.w), -g));
+    return make_float4(fmaf(g * xx.x, rcp_approx_sub(r.x), -g), fmaf(g * xx.y, rcp_approx_sub(r.y), -g),
+                       fmaf(g * xx.z, rcp_approx_sub(r.z), -g), fmaf(g * xx.w, rcp_approx_sub(r.w), -g));
 }
 
 template <int INNER4, int NBOX>

@@ -837,10 +837,12 @@ __global__ void __launch_bounds__(256) k_philox_raw(uint32_t* __restrict__ out, 
 // ---------------------------------------------------------------------------
 // host-side dispatch
 // ---------------------------------------------------------------------------
+// The VEC kernels walk whole packs of a row, so E % VN == 0 is needed whatever the modes are: with every operand
+// SCALAR nothing else would stop a pack past E (or the dropped tail of E / VN packs).
 template <typename T>
 static bool vec_ok(const Operand<T>& o, int64_t E) {
-    if (o.p == nullptr || o.mode == ZS_SCALAR) return true;
-    return aligned16(o.p) && (E % Pack<T>::N == 0);
+    if (E % Pack<T>::N != 0) return false;
+    return o.p == nullptr || o.mode == ZS_SCALAR || aligned16(o.p);
 }
 
 template <typename T, typename Op, int LPR>
