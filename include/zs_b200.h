@@ -42,7 +42,8 @@ extern "C" {
 #endif
 
 /* 3: zs_allreduce_sum_peer takes (extra_src, extra_index); new: zs_allreduce_sum_nvls, zs_iw_bernoulli_fused_loss,
- *    zs_debug_set_latent_fwd; later additions (compatible): zs_poisson_*, zs_iw_poisson_fused[_loss].  2: device-side Philox state, handle-based host step, flags argument of the fused kernel. */
+ *    zs_debug_set_latent_fwd; later additions (compatible): zs_poisson_*, zs_iw_poisson_fused[_loss], zs_beta_sample,
+ *    ZS_FAM_BETA of zs_locscale_logprob_fwd/bwd.  2: device-side Philox state, handle-based host step, flags argument of the fused kernel. */
 #define ZS_ABI_VERSION 3
 
 typedef void* zs_stream_t; /* cudaStream_t */
@@ -50,8 +51,8 @@ typedef void* zs_stream_t; /* cudaStream_t */
 enum { ZS_F32 = 0, ZS_F64 = 1 };
 enum { ZS_FULL = 0, ZS_KBCAST = 1, ZS_SCALAR = 2 };
 enum { ZS_EST_SGVB = 0, ZS_EST_VIMCO = 1, ZS_EST_ELBO = 2 };
-/* location-scale families of the zs_locscale_* entry points */
-enum { ZS_FAM_LOGISTIC = 1, ZS_FAM_LAPLACE = 2, ZS_FAM_UNIFORM = 3 };
+/* location-scale families of the zs_locscale_* entry points (ZS_FAM_BETA: the log-density entry points only) */
+enum { ZS_FAM_LOGISTIC = 1, ZS_FAM_LAPLACE = 2, ZS_FAM_UNIFORM = 3, ZS_FAM_BETA = 4 };
 
 enum {
     ZS_OK = 0,
@@ -144,7 +145,11 @@ int zs_normal_logprob_bwd(int dtype, void* dx, void* dmean, void* dstd, const vo
  * ZS_FAM_UNIFORM (Uniform, zhusuan/distributions/uniform.py:51-83): _sample draws u ~ U[0,1) (torch.rand, :63-66) and
  * returns loc + scale * u (pass loc = low, scale = high - low; or 0 / 1 for the unit draw the reference caches);
  * _logprob_* take loc = LOW and scale = HIGH: -log(high - low) on [low, high), -inf outside
- * (torch.distributions.Uniform.log_prob, :81), d/dlow = g/(high - low), d/dhigh = -g/(high - low), d/dx = 0. */
+ * (torch.distributions.Uniform.log_prob, :81), d/dlow = g/(high - low), d/dhigh = -g/(high - low), d/dx = 0.
+ * ZS_FAM_BETA (Beta, the reference's zhusuan/distributions/beta.py via torch.distributions.Beta): _logprob_* only, with
+ * loc = ALPHA and scale = BETA: xlogy(alpha - 1, x) + xlogy(beta - 1, 1 - x) + lgamma(alpha + beta)
+ * - (lgamma(alpha) + lgamma(beta)), and torch's autograd of it (dalpha = xlogy(g, x) + g psi(alpha + beta)
+ * - g psi(alpha), likewise dbeta with 1 - x; dx = g (alpha - 1) / x - g (beta - 1) / (1 - x)).  Samples: zs_beta_sample. */
 int zs_locscale_sample(int dtype, int family, void* z, const void* loc, int loc_mode, const void* scale, int scale_mode,
                        const void* u_in, int64_t K, int64_t N, uint64_t seed, uint64_t offset, void* rng_state,
                        void* rng_snapshot, zs_stream_t stream);
@@ -196,6 +201,17 @@ int zs_poisson_logpmf_fwd(int dtype, void* out, const void* x, int x_mode, const
 /* drate = g * (x / rate - 1); the count has no gradient.  drate may be NULL (nothing to do).                          */
 int zs_poisson_logpmf_bwd(int dtype, void* drate, const void* g, const void* x, int x_mode, const void* rate,
                           int rate_mode, int64_t K, int64_t M, int64_t E, zs_stream_t stream);
+
+/* ---- Beta stochastic node ---------------------------------------------------------------------------------
+ * zs_beta_sample: out[K,N] = Beta(alpha, beta) samples; alpha and beta modes ZS_FULL|ZS_KBCAST|ZS_SCALAR.  As torch's
+ *   CPU Dirichlet sampler: two Marsaglia-Tsang gamma draws (shape < 1 boosted), in double, G_alpha / (G_alpha +
+ *   G_beta) clamped to [smallest normal of the dtype, nextafter(1, 0)].  Element i takes its words from the Philox
+ *   groups (counter i | (j << 48), at most 65 groups) of the position (seed, offset [+ rng_state]), as
+ *   zs_poisson_sample: independent of the launch geometry.  Needs K*N < 2^48.  Parameters are not validated: an alpha
+ *   or beta that is not positive and finite (0, negative, infinite, NaN) gives NaN.  The log-density is
+ *   zs_locscale_logprob_fwd/bwd with ZS_FAM_BETA.                                                                */
+int zs_beta_sample(int dtype, void* out, const void* alpha, int alpha_mode, const void* beta, int beta_mode, int64_t K,
+                   int64_t N, uint64_t seed, uint64_t offset, void* rng_state, zs_stream_t stream);
 
 /* ---- fused latent-node kernels (zs_latent.cu) -------------------------------
  * Forward: z ~ q (Philox or injected noise), log q(z) and log p(z) under the prior, both summed over

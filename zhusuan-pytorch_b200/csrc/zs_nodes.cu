@@ -1,4 +1,4 @@
-// Stochastic-node kernels: sample and log-prob (forward / backward) for Normal, Bernoulli and Poisson
+// Stochastic-node kernels: sample and log-prob (forward / backward) for Normal, Bernoulli, Poisson and Beta
 // over the [K, M, E] particle-row view described in include/zs_b200.h.
 //
 // Replaces (reference file:line):
@@ -14,6 +14,8 @@
 #include "zs_common.cuh"
 
 #include <cooperative_groups.h>
+#include <float.h>
+#include <type_traits>
 #include "zs_philox.cuh"
 
 namespace zs {
@@ -218,17 +220,90 @@ struct PoissonOp {
     }
 };
 
+// digamma, restating ATen's calc_digamma (ATen/native/Math.h, from Cephes): the reflection for x < 0, the recurrence
+// up to 10, PSI_10 at exactly 10, the asymptotic series above.  The float form stays in float except for the
+// reflection term, as ATen's CPU float version does.
+template <typename T>
+__device__ __forceinline__ T digamma_t(T x) {
+    if (x == T(0)) return copysign((T)INFINITY, -x);
+    T refl = T(0);
+    if (x < T(0)) {
+        if (x == trunc(x)) return (T)NAN;
+        double q;
+        const double r = modf((double)x, &q);
+        refl = (T)(3.141592653589793 / ::tan(3.141592653589793 * r));
+        x = T(1) - x;
+    }
+    T result = T(0);
+    while (x < T(10)) {
+        result -= T(1) / x;
+        x += T(1);
+    }
+    if (x == T(10)) return (result + (T)2.25175258906672110764) - refl;
+    T y = T(0);
+    if (x < (T)1.0e17) {
+        const T z = T(1) / (x * x);
+        T p = (T)8.33333333333333333333E-2;
+        p = p * z + (T)-2.10927960927960927961E-2;
+        p = p * z + (T)7.57575757575757575758E-3;
+        p = p * z + (T)-4.16666666666666666667E-3;
+        p = p * z + (T)3.96825396825396825397E-3;
+        p = p * z + (T)-8.33333333333333333333E-3;
+        p = p * z + (T)8.33333333333333333333E-2;
+        y = z * p;
+    }
+    return (((result + Real<T>::log(x)) - (T(0.5) / x)) - y) - refl;
+}
+
+// Beta(alpha, beta): torch.distributions.Beta.log_prob, which goes through Dirichlet.log_prob on stack([x, 1 - x]):
+//   xlogy(alpha - 1, x) + xlogy(beta - 1, 1 - x) + lgamma(alpha + beta) - (lgamma(alpha) + lgamma(beta))
+// with 1 - x rounded in the operand dtype first, as torch does.  Gradients are torch's autograd of that expression:
+//   dx = g (alpha - 1) / x - g (beta - 1) / (1 - x),  dalpha = xlogy(g, x) + g psi(alpha + beta) - g psi(alpha)
+// with xlogy's rule that drops the log where alpha - 1 == 0 and x <= 0 (and likewise for beta and 1 - x).
+// The parameter-only terms (the two lgamma sums; the three psi values) come in as arguments, so that a caller holding
+// them for many elements (ScalarB, k_kreduce_bwd_hoisted) computes bit-identically to term / grad.
+template <typename T>
+struct BetaOp {
+    static __device__ __forceinline__ T xlogy(T c, T v) {
+        if (isnan(v)) return v;
+        return c == T(0) ? T(0) : c * Real<T>::log(v);
+    }
+    static __device__ __forceinline__ T lgab(T a, T b) { return lgamma_t(a + b); }
+    static __device__ __forceinline__ T lga_lgb(T a, T b) { return lgamma_t(a) + lgamma_t(b); }
+    static __device__ __forceinline__ T term_h(T x, T a, T b, T lab, T la_lb) {
+        const T s = xlogy(a - T(1), x) + xlogy(b - T(1), T(1) - x);
+        return (s + lab) - la_lb;
+    }
+    static __device__ __forceinline__ T term(T x, T a, T b) { return term_h(x, a, b, lgab(a, b), lga_lgb(a, b)); }
+    static __device__ __forceinline__ T finish(T acc) { return acc; }
+    template <bool NEED_X>
+    static __device__ __forceinline__ void grad_h(T g, T x, T a, T b, T psab, T psa, T psb, T& dx, T& da, T& db) {
+        const T am1 = a - T(1), bm1 = b - T(1), y = T(1) - x;
+        dx = NEED_X ? (g * am1) / x - (g * bm1) / y : T(0);
+        const T lx = (am1 == T(0) && x <= T(0)) ? T(0) : xlogy(g, x);
+        const T ly = (bm1 == T(0) && y <= T(0)) ? T(0) : xlogy(g, y);
+        const T gs = g * psab;
+        da = (lx + gs) - g * psa;
+        db = (ly + gs) - g * psb;
+    }
+    template <bool NEED_X>
+    static __device__ __forceinline__ void grad(T g, T x, T a, T b, T& dx, T& da, T& db) {
+        grad_h<NEED_X>(g, x, a, b, digamma_t(a + b), digamma_t(a), digamma_t(b), dx, da, db);
+    }
+};
+
 // ---------------------------------------------------------------------------
 // A SCALAR (or absent) second parameter is the same for every element of the launch: whatever the op derives from it
 // alone is computed once per thread, not once per element.  For the Normal op that is log(std), exp(-2 log std) and
 // 1/std -- the BNN likelihood of bnn_vi.py:55-60 (mean [K, batch], ONE logstd) otherwise spends three transcendentals
 // per element on a constant and is issue-bound at 0.3-0.4 of the HBM roofline (profiles/r1_bnn_kernels.json).
 // Same expressions in the same order as Op::term / Op::grad, so results are bit-identical.
+// `a_` / `a_scalar`: the first parameter, for ops whose parameter-only terms need both (Beta, when both are SCALAR).
 // ---------------------------------------------------------------------------
 template <typename T, typename Op>
 struct ScalarB {
     T b;
-    __device__ __forceinline__ explicit ScalarB(T b_) : b(b_) {}
+    __device__ __forceinline__ ScalarB(T b_, T /*a_*/, bool /*a_scalar*/) : b(b_) {}
     __device__ __forceinline__ T term(T x, T a) const { return Op::term(x, a, b); }
     template <bool NEED_X>
     __device__ __forceinline__ void grad(T g, T x, T a, T& dx, T& da, T& db) const {
@@ -238,7 +313,7 @@ struct ScalarB {
 template <typename T>
 struct ScalarB<T, NormalOp<T>> {
     T std, logstd, prec;
-    __device__ __forceinline__ explicit ScalarB(T b_) : std(b_) {
+    __device__ __forceinline__ ScalarB(T b_, T /*a_*/, bool /*a_scalar*/) : std(b_) {
         logstd = Real<T>::log(b_);
         prec = Real<T>::exp(T(-2) * logstd);
     }
@@ -255,6 +330,31 @@ struct ScalarB<T, NormalOp<T>> {
         T dprec = -(g * (d * d)) * T(0.5);
         T dlogstd = -g + (dprec * prec) * T(-2);
         dstd = dlogstd / std;
+    }
+};
+// Beta with SCALAR alpha AND beta (the prior of a Beta node): the lgamma sums and the three psi values are the same for
+// every element, so they are formed once per thread.  A FULL / KBCAST alpha keeps the per-element path.
+template <typename T>
+struct ScalarB<T, BetaOp<T>> {
+    T b;
+    bool hoisted;
+    T lab, la_lb, psab, psa, psb;
+    __device__ __forceinline__ ScalarB(T b_, T a_, bool a_scalar) : b(b_), hoisted(a_scalar) {
+        if (hoisted) {
+            lab = BetaOp<T>::lgab(a_, b_);
+            la_lb = BetaOp<T>::lga_lgb(a_, b_);
+            psab = digamma_t(a_ + b_);
+            psa = digamma_t(a_);
+            psb = digamma_t(b_);
+        }
+    }
+    __device__ __forceinline__ T term(T x, T a) const {
+        return hoisted ? BetaOp<T>::term_h(x, a, b, lab, la_lb) : BetaOp<T>::term(x, a, b);
+    }
+    template <bool NEED_X>
+    __device__ __forceinline__ void grad(T g, T x, T a, T& dx, T& da, T& db) const {
+        if (hoisted) BetaOp<T>::template grad_h<NEED_X>(g, x, a, b, psab, psa, psb, dx, da, db);
+        else BetaOp<T>::template grad<NEED_X>(g, x, a, b, dx, da, db);
     }
 };
 
@@ -274,7 +374,7 @@ __global__ void __launch_bounds__(256) k_rows_fwd(T* __restrict__ out, Operand<T
     const T bs = (b.p != nullptr && b.mode == ZS_SCALAR) ? b.p[0] : T(0);
     const bool hasb = b.p != nullptr;
     const bool bsc = !hasb || b.mode == ZS_SCALAR;
-    const ScalarB<T, Op> sb(bs);
+    const ScalarB<T, Op> sb(bs, as, a.mode == ZS_SCALAR);
 
     for (int64_t base = 0; base < R; base += ngrp) {
         const int64_t r = base + grp;
@@ -366,7 +466,7 @@ __global__ void __cluster_dims__(ROWC, 1, 1) __launch_bounds__(256)
     const T bs = (b.p != nullptr && b.mode == ZS_SCALAR) ? b.p[0] : T(0);
     const bool hasb = b.p != nullptr;
     const bool bsc = !hasb || b.mode == ZS_SCALAR;
-    const ScalarB<T, Op> sb(bs);
+    const ScalarB<T, Op> sb(bs, as, a.mode == ZS_SCALAR);
     // contiguous segment of this CTA, a multiple of the pack width
     const int64_t per = ((E + (int64_t)ROWC * VN - 1) / ((int64_t)ROWC * VN)) * VN;
     const int64_t lo = (int64_t)rank * per, hi = lo + per < E ? lo + per : E;
@@ -445,7 +545,7 @@ __global__ void __launch_bounds__(256) k_rows_bwd(T* __restrict__ dx, T* __restr
     const T bs = (b.p != nullptr && b.mode == ZS_SCALAR) ? b.p[0] : T(0);
     const bool hasb = b.p != nullptr;
     const bool bsc = !hasb || b.mode == ZS_SCALAR;
-    const ScalarB<T, Op> sb(bs);
+    const ScalarB<T, Op> sb(bs, as, a.mode == ZS_SCALAR);
 
     for (int64_t r = grp; r < R; r += ngrp) {
         const int64_t m = r % M;
@@ -541,7 +641,7 @@ __global__ void __launch_bounds__(KR_X* KR_Y) k_kreduce_bwd(T* __restrict__ dx, 
         const T as = a.mode == ZS_SCALAR ? a.p[0] : T(0);
         const T bs = (hasb && b.mode == ZS_SCALAR) ? b.p[0] : T(0);
         const bool bsc = !hasb || b.mode == ZS_SCALAR;
-        const ScalarB<T, Op> sbp(bs);
+        const ScalarB<T, Op> sbp(bs, as, a.mode == ZS_SCALAR);
 #pragma unroll 4
         for (int64_t k = threadIdx.y; k < K; k += KR_Y) {
             const int64_t f = k * ME + n;
@@ -586,6 +686,59 @@ __global__ void __launch_bounds__(KR_X* KR_Y) k_kreduce_bwd(T* __restrict__ dx, 
         if (dx && x.mode == ZS_KBCAST) dx[n] = tx;
         if (da && a.mode == ZS_KBCAST) da[n] = ta;
         if (db && hasb && b.mode == ZS_KBCAST) db[n] = tb;
+    }
+}
+
+// k_kreduce_bwd for the Beta op when neither parameter is FULL (the variational posterior of a Beta node: alpha and
+// beta KBCAST over the K particles): psi(alpha + beta), psi(alpha) and psi(beta) depend on n only, so each thread forms
+// them once, outside its particle loop, instead of once per particle.  Same block shape and fixed-order sum as
+// k_kreduce_bwd; a kernel of its own so that the other ops' k_kreduce_bwd instantiations are untouched.
+template <typename T>
+__global__ void __launch_bounds__(KR_X* KR_Y) k_kreduce_bwd_beta(T* __restrict__ dx, T* __restrict__ da,
+                                                                  T* __restrict__ db, const T* __restrict__ g,
+                                                                  Operand<T> x, Operand<T> a, Operand<T> b, int64_t K,
+                                                                  int64_t M, int64_t E) {
+    const int64_t ME = M * E;
+    const int64_t n = (int64_t)blockIdx.x * KR_X + threadIdx.x;
+    const bool valid = n < ME;
+    const int64_t m = valid ? n / E : 0;
+    T sx = T(0), sa = T(0), sb = T(0);
+    if (valid) {
+        const T xs = x.mode == ZS_SCALAR ? x.p[0] : T(0);
+        const T av = a.mode == ZS_KBCAST ? a.p[n] : a.p[0];
+        const T bv = b.mode == ZS_KBCAST ? b.p[n] : b.p[0];
+        const T psab = digamma_t(av + bv), psa = digamma_t(av), psb = digamma_t(bv);
+#pragma unroll 4
+        for (int64_t k = threadIdx.y; k < K; k += KR_Y) {
+            const int64_t f = k * ME + n;
+            const T gv = g[k * M + m];
+            const T xv = x.mode == ZS_FULL ? x.p[f] : (x.mode == ZS_KBCAST ? x.p[n] : xs);
+            T ox, oa, ob;
+            if (dx) BetaOp<T>::template grad_h<true>(gv, xv, av, bv, psab, psa, psb, ox, oa, ob);
+            else BetaOp<T>::template grad_h<false>(gv, xv, av, bv, psab, psa, psb, ox, oa, ob);
+            if (dx) {
+                if (x.mode == ZS_FULL) dx[f] = ox; else sx += ox;
+            }
+            sa += oa;
+            sb += ob;
+        }
+    }
+    __shared__ T red[3][KR_Y][KR_X + 1];
+    red[0][threadIdx.y][threadIdx.x] = sx;
+    red[1][threadIdx.y][threadIdx.x] = sa;
+    red[2][threadIdx.y][threadIdx.x] = sb;
+    __syncthreads();
+    if (threadIdx.y == 0 && valid) {
+        T tx = T(0), ta = T(0), tb = T(0);
+#pragma unroll
+        for (int s = 0; s < KR_Y; ++s) {
+            tx += red[0][s][threadIdx.x];
+            ta += red[1][s][threadIdx.x];
+            tb += red[2][s][threadIdx.x];
+        }
+        if (dx && x.mode == ZS_KBCAST) dx[n] = tx;
+        if (da && a.mode == ZS_KBCAST) da[n] = ta;
+        if (db && b.mode == ZS_KBCAST) db[n] = tb;
     }
 }
 
@@ -803,6 +956,78 @@ __global__ void __launch_bounds__(256) k_poisson_sample(T* __restrict__ out, con
     }
 }
 
+// Beta(alpha, beta) samples (torch.distributions.Beta.sample, which the reference's beta.py calls), drawn as torch's
+// CPU Dirichlet sampler does: G_alpha then G_beta with ATen's sample_gamma (Marsaglia and Tsang, "A simple method for
+// generating gamma variables", 2000; shape < 1 boosted by (1 - u)^(1/shape) and shape + 1), each clamped below at
+// DBL_MIN, and G_alpha / (G_alpha + G_beta) rounded to the output dtype and clamped to [smallest normal, nextafter(1, 0)]:
+// never 0 or 1, so log_prob at a sample is finite.  Double arithmetic for both dtypes.  Element i reads its words as
+// the Poisson sampler does (counter i | (j << 48)); a standard normal is Box-Muller on two words, cos branch.  A gamma
+// trial takes three words (two for the normal, one uniform) and is accepted with probability above 0.95 for the boosted
+// shapes >= 1; a normal with 1 + c x <= 0 is redrawn (two words).  The loop stops after BETA_MAX_WORDS words for the
+// element, and a gamma draw that meets the cap returns its v = 1 point scale * d.  Meeting it takes at least 84 attempts
+// with at most two acceptances among them: P < C(84, 2) 0.05^82 < 1e-100.  Parameters are not validated: alpha or beta
+// that is not positive and finite (zero, negative, infinite, NaN) gives NaN.
+constexpr int BETA_MAX_WORDS = 256;
+
+__device__ __forceinline__ double philox_words_normal(PhiloxWords& u) {
+    const double u1 = 1.0 - u.next();  // (0, 1]
+    const double u2 = u.next();
+    return ::sqrt(-2.0 * ::log(u1)) * ::cos(6.283185307179586 * u2);
+}
+
+__device__ double gamma_draw(double alpha, PhiloxWords& u) {
+    double scale = 1.0;
+    if (alpha < 1.0) {
+        scale *= ::pow(1.0 - u.next(), 1.0 / alpha);
+        alpha += 1.0;
+    }
+    // ATen's constants are float literals promoted to double
+    const double d = alpha - (double)(1.0f / 3.0f);
+    const double c = 1.0 / ::sqrt(9.0 * d);
+    while (u.used < BETA_MAX_WORDS) {
+        const double x = philox_words_normal(u);
+        const double y = 1.0 + c * x;
+        if (y <= 0.0) continue;
+        const double v = y * y * y;
+        const double U = 1.0 - u.next();
+        const double xx = x * x;
+        if (U < 1.0 - (double)0.0331f * xx * xx) return scale * d * v;
+        if (::log(U) < 0.5 * xx + d * (1.0 - v + ::log(v))) return scale * d * v;
+    }
+    return scale * d;
+}
+
+template <typename T>
+__device__ __forceinline__ T beta_clamp(double r);
+template <>
+__device__ __forceinline__ float beta_clamp<float>(double r) {
+    return fminf(fmaxf((float)r, FLT_MIN), 0.99999994f);  // nextafterf(1, 0) = 1 - 2^-24
+}
+template <>
+__device__ __forceinline__ double beta_clamp<double>(double r) {
+    return fmin(fmax(r, DBL_MIN), 0.99999999999999989);  // nextafter(1, 0) = 1 - 2^-53
+}
+
+template <typename T>
+__global__ void __launch_bounds__(256) k_beta_sample(T* __restrict__ out, const T* __restrict__ alpha, int am,
+                                                     const T* __restrict__ beta, int bm, int64_t K, int64_t N,
+                                                     uint64_t seed, uint64_t offset, unsigned long long* rs) {
+    offset = rng_acquire(offset, rs, nullptr, true);
+    const int64_t total = K * N;
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (int64_t)gridDim.x * blockDim.x) {
+        const double av = (double)(am == ZS_FULL ? alpha[i] : (am == ZS_KBCAST ? alpha[i % N] : alpha[0]));
+        const double bv = (double)(bm == ZS_FULL ? beta[i] : (bm == ZS_KBCAST ? beta[i % N] : beta[0]));
+        if (!(av > 0.0 && bv > 0.0 && av < INFINITY && bv < INFINITY)) {
+            out[i] = (T)NAN;
+            continue;
+        }
+        PhiloxWords u{(uint64_t)i, offset, seed, {0u, 0u, 0u, 0u}, 0};
+        const double ga = fmax(gamma_draw(av, u), DBL_MIN);
+        const double gb = fmax(gamma_draw(bv, u), DBL_MIN);
+        out[i] = beta_clamp<T>(ga / (ga + gb));
+    }
+}
+
 template <typename T>
 __global__ void __launch_bounds__(256) k_philox_fill(T* __restrict__ out, int64_t n, T mean, T std, int normal,
                                                      uint64_t seed, uint64_t offset, unsigned long long* rs) {
@@ -914,6 +1139,13 @@ static int dispatch_bwd(T* dx, T* da, T* db, const T* g, Operand<T> x, Operand<T
         dim3 block(KR_X, KR_Y);
         const int64_t grid = (ME + KR_X - 1) / KR_X;
         ZS_REQUIRE(grid < (int64_t)2147483647, ZS_ERR_UNSUPPORTED);
+        if constexpr (std::is_same<Op, BetaOp<T>>::value) {
+            if (a.mode != ZS_FULL && b.mode != ZS_FULL) {
+                k_kreduce_bwd_beta<T><<<(unsigned)grid, block, 0, st>>>(dx, da, db, g, x, a, b, K, M, E);
+                ZS_LAUNCH_CHECK("k_kreduce_bwd_beta");
+                return ZS_OK;
+            }
+        }
         k_kreduce_bwd<T, Op><<<(unsigned)grid, block, 0, st>>>(dx, da, db, g, x, a, b, K, M, E);
         ZS_LAUNCH_CHECK("k_kreduce_bwd");
         return ZS_OK;
@@ -1174,8 +1406,14 @@ int zs_locscale_logprob_fwd(int dtype, int family, void* out, const void* x, int
                             const void* scale, int scale_mode, int64_t K, int64_t M, int64_t E, zs_stream_t stream) {
     ZS_REQUIRE(out && x && loc && scale && K >= 0 && M >= 0 && E >= 1, ZS_ERR_ARG);
     ZS_REQUIRE(valid_mode(x_mode) && valid_mode(loc_mode) && valid_mode(scale_mode), ZS_ERR_ARG);
-    ZS_REQUIRE(family == ZS_FAM_LOGISTIC || family == ZS_FAM_LAPLACE || family == ZS_FAM_UNIFORM, ZS_ERR_ARG);
+    ZS_REQUIRE(family == ZS_FAM_LOGISTIC || family == ZS_FAM_LAPLACE || family == ZS_FAM_UNIFORM ||
+                   family == ZS_FAM_BETA,
+               ZS_ERR_ARG);
     ZS_DTYPE_SWITCH(dtype, {
+        if (family == ZS_FAM_BETA)  // loc = alpha, scale = beta
+            return dispatch_rows_fwd<T, BetaOp<T>>((T*)out, Operand<T>{(const T*)x, x_mode},
+                                                   Operand<T>{(const T*)loc, loc_mode},
+                                                   Operand<T>{(const T*)scale, scale_mode}, K, M, E, as_stream(stream));
         if (family == ZS_FAM_LOGISTIC)
             return dispatch_rows_fwd<T, LogisticOp<T>>((T*)out, Operand<T>{(const T*)x, x_mode},
                                                        Operand<T>{(const T*)loc, loc_mode},
@@ -1195,9 +1433,15 @@ int zs_locscale_logprob_bwd(int dtype, int family, void* dx, void* dloc, void* d
                             int64_t M, int64_t E, zs_stream_t stream) {
     ZS_REQUIRE(g && x && loc && scale && K >= 0 && M >= 0 && E >= 1, ZS_ERR_ARG);
     ZS_REQUIRE(valid_mode(x_mode) && valid_mode(loc_mode) && valid_mode(scale_mode), ZS_ERR_ARG);
-    ZS_REQUIRE(family == ZS_FAM_LOGISTIC || family == ZS_FAM_LAPLACE || family == ZS_FAM_UNIFORM, ZS_ERR_ARG);
+    ZS_REQUIRE(family == ZS_FAM_LOGISTIC || family == ZS_FAM_LAPLACE || family == ZS_FAM_UNIFORM ||
+                   family == ZS_FAM_BETA,
+               ZS_ERR_ARG);
     if (!dx && !dloc && !dscale) return ZS_OK;
     ZS_DTYPE_SWITCH(dtype, {
+        if (family == ZS_FAM_BETA)
+            return dispatch_bwd<T, BetaOp<T>>((T*)dx, (T*)dloc, (T*)dscale, (const T*)g, Operand<T>{(const T*)x, x_mode},
+                                              Operand<T>{(const T*)loc, loc_mode},
+                                              Operand<T>{(const T*)scale, scale_mode}, K, M, E, as_stream(stream));
         if (family == ZS_FAM_LOGISTIC)
             return dispatch_bwd<T, LogisticOp<T>>((T*)dx, (T*)dloc, (T*)dscale, (const T*)g, Operand<T>{(const T*)x, x_mode},
                                                   Operand<T>{(const T*)loc, loc_mode},
@@ -1273,6 +1517,21 @@ int zs_poisson_logpmf_bwd(int dtype, void* drate, const void* g, const void* x, 
                                              Operand<T>{(const T*)x, x_mode}, Operand<T>{(const T*)rate, rate_mode},
                                              Operand<T>{nullptr, ZS_SCALAR}, K, M, E, as_stream(stream));
     })
+}
+
+/* ---- Beta stochastic node (log-density: zs_locscale_logprob_* with ZS_FAM_BETA) ------------------------------ */
+int zs_beta_sample(int dtype, void* out, const void* alpha, int alpha_mode, const void* beta, int beta_mode, int64_t K,
+                   int64_t N, uint64_t seed, uint64_t offset, void* rng_state, zs_stream_t stream) {
+    ZS_REQUIRE(out && alpha && beta && K >= 0 && N >= 0 && valid_mode(alpha_mode) && valid_mode(beta_mode), ZS_ERR_ARG);
+    if (K * N == 0) return ZS_OK;
+    ZS_REQUIRE(K * N < ((int64_t)1 << 48), ZS_ERR_UNSUPPORTED);  // element index below the group bits of the counter
+    const int grid = grid_for(K * N, 256);
+    ZS_DTYPE_SWITCH(dtype, {
+        k_beta_sample<T><<<grid, 256, 0, as_stream(stream)>>>((T*)out, (const T*)alpha, alpha_mode, (const T*)beta,
+                                                              beta_mode, K, N, seed, offset, rs_ptr(rng_state));
+    })
+    ZS_LAUNCH_CHECK("k_beta_sample");
+    return ZS_OK;
 }
 
 }  // extern "C"

@@ -66,6 +66,7 @@ def _declare(lib):
         "zs_locscale_logprob_fwd": (i32, [i32, i32, vp, vp, i32, vp, i32, vp, i32, i64, i64, i64, vp]),
         "zs_locscale_logprob_bwd": (i32, [i32, i32, vp, vp, vp, vp, vp, i32, vp, i32, vp, i32, i64, i64, i64, vp]),
         "zs_poisson_sample": (i32, [i32, vp, vp, i32, i64, i64, u64, u64, vp, vp]),
+        "zs_beta_sample": (i32, [i32, vp, vp, i32, vp, i32, i64, i64, u64, u64, vp, vp]),
         "zs_poisson_logpmf_fwd": (i32, [i32, vp, vp, i32, vp, i32, i64, i64, i64, vp]),
         "zs_poisson_logpmf_bwd": (i32, [i32, vp, vp, vp, i32, vp, i32, i64, i64, i64, vp]),
         "zs_iw_poisson_fused": (i32, [i32, vp, vp, vp, vp, vp, vp, vp, vp, vp, i64, i64, i64, dbl, i32, vp]),
@@ -399,8 +400,21 @@ def poisson_logpmf_bwd(g, x, xm, rate, rm, K, M, E):
     return drate
 
 
+# ----------------------------------------------------------------------------- Beta
+def beta_sample(alpha, am, beta, bm, K, N, seed=0, offset=0, rng_state=None):
+    """zs_beta_sample: [K, N] Beta(alpha, beta) samples; the log-density is locscale_logprob_* with FAM_BETA."""
+    dt, dev = alpha.dtype, alpha.device
+    _chk(dev, dt, alpha=alpha, beta=beta)
+    _chk_state(dev, rng_state=rng_state)
+    out = torch.empty((K, N), dtype=dt, device=dev)
+    _go("zs_beta_sample", dev, dtype_code(dt), _ptr(out), _ptr(alpha), am, _ptr(beta), bm, K, N, seed, offset,
+        _ptr(rng_state))
+    return out
+
+
 # ----------------------------------------------------------------------------- Logistic / Laplace
-FAM_LOGISTIC, FAM_LAPLACE, FAM_UNIFORM = 1, 2, 3
+# FAM_BETA: the log-density entry points only (loc = alpha, scale = beta); its sampler is beta_sample
+FAM_LOGISTIC, FAM_LAPLACE, FAM_UNIFORM, FAM_BETA = 1, 2, 3, 4
 
 
 def locscale_sample(family, loc, loc_mode, scale, scale_mode, K, N, u_in=None, seed=0, offset=0, rng_state=None,

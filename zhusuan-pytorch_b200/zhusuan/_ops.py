@@ -707,6 +707,29 @@ def poisson_sample(rate, n_samples):
 
 
 # --------------------------------------------------------------------------------------------
+# Beta (log-density: locscale_log_prob with FAM_BETA)
+# --------------------------------------------------------------------------------------------
+def beta_sample(alpha, beta, n_samples):
+    """Beta._sample (torch.distributions.Beta.sample, which the reference's beta.py calls): [n_samples] + the
+    broadcast shape of alpha and beta (no leading axis for n_samples 1), drawn in-kernel; no gradient."""
+    home = alpha.device
+    # uploaded outside no_grad: a memoised upload is reused by the log-density, which needs its autograd edge
+    alpha, beta = to_compute(alpha).detach(), to_compute(beta).detach()
+    with torch.no_grad():
+        base = tuple(_bshapes(alpha.shape, beta.shape))
+        alpha, beta = alpha.expand(base).contiguous(), beta.expand(base).contiguous()
+        K = int(n_samples)
+        out_shape = ((K,) if K > 1 else ()) + base
+        N = _prod(base)
+        if N == 0:
+            return back_home(torch.zeros(out_shape, dtype=alpha.dtype, device=alpha.device), home)
+        kw, _ = _draw_kwargs(alpha.device, None)
+        mode = KBCAST if K > 1 else FULL
+        out = be.beta_sample(alpha, mode, beta, mode, K, N, **kw)
+    return back_home(out.reshape(out_shape), home)
+
+
+# --------------------------------------------------------------------------------------------
 # Categorical (not in the reference; see distributions/categorical.py)
 # --------------------------------------------------------------------------------------------
 class _CategoricalLogPmf(torch.autograd.Function):

@@ -3,14 +3,14 @@
 Same attributes (`_nodes`, `_cache`, `_observed`, `_device`), properties and methods as the
 reference (:72-240): `observe`, `stochastic_node` / `sn` / `snode`, the per-distribution aliases of
 the hot-path distributions, `log_joint` / `_log_joint`.  Normal, Bernoulli, Categorical, Logistic, Laplace,
-Uniform and Poisson are registered: the other aliases of the reference (beta, gamma, ...) wrap
+Uniform, Poisson and Beta are registered: the other aliases of the reference (gamma, exponential, studentT) wrap
 torch.distributions and are outside the accelerated path.
 """
 import torch
 import torch.nn as nn
 
 from zhusuan.framework.stochastic_tensor import StochasticTensor
-from zhusuan.distributions import Distribution, Normal, Bernoulli, Categorical, Logistic, Laplace, Uniform, Poisson
+from zhusuan.distributions import Distribution, Normal, Bernoulli, Categorical, Logistic, Laplace, Uniform, Poisson, Beta
 
 __all__ = ['BayesianNet']
 
@@ -22,9 +22,10 @@ name_mapping = {
     "Laplace": Laplace,
     "Uniform": Uniform,
     "Poisson": Poisson,
+    "Beta": Beta,
 }
 
-_OUT_OF_SCOPE = ("Beta", "Exponential", "Gamma", "StudentT")
+_OUT_OF_SCOPE = ("Exponential", "Gamma", "StudentT")
 
 
 class BayesianNet(nn.Module):
@@ -78,8 +79,8 @@ class BayesianNet(nn.Module):
         if isinstance(distribution, str):
             if distribution not in name_mapping:
                 if distribution in _OUT_OF_SCOPE:
-                    raise NotImplementedError(
-                        "%s is outside the B200 hot path (Normal, Bernoulli, Categorical)" % distribution)
+                    raise NotImplementedError("%s is outside the B200 hot path (registered: %s)"
+                                              % (distribution, ", ".join(name_mapping)))
                 raise KeyError(distribution)
             dist = name_mapping[distribution](device=self.device, **kwargs)
         elif isinstance(distribution, Distribution):
@@ -124,6 +125,13 @@ class BayesianNet(nn.Module):
             raise ValueError("name of stochastic_node must be str")
         dist = Poisson(rate=rate, dtype=dtype, is_continuous=is_continuous, group_ndims=group_ndims,
                        device=self.device, **kwargs)
+        return self._register(name, dist, n_samples, kwargs)
+
+    def beta(self, name, alpha, beta, dtype=None, is_continuous=True, group_ndims=0, n_samples=None, **kwargs):
+        if not isinstance(name, str):
+            raise ValueError("name of stochastic_node must be str")
+        dist = Beta(alpha=alpha, beta=beta, dtype=dtype, is_continuous=is_continuous, group_ndims=group_ndims,
+                    device=self.device, **kwargs)
         return self._register(name, dist, n_samples, kwargs)
 
     def laplace(self, name, loc, scale, dtype=None, is_continuous=True, group_ndims=0, n_samples=None, **kwargs):
