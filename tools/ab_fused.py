@@ -1,9 +1,11 @@
 """A/B timing of zs_iw_bernoulli_fused between builds of the library, interleaved in one process so
-box-to-box and clock drift cancel.  Usage: ab_fused.py name=path.so [name=path.so ...]   (GPU box only)"""
+box-to-box and clock drift cancel.  Usage: ab_fused.py name=path.so [name=path.so ...]   (GPU box only)
+AB_B (default 1024) and AB_K (default 50) set the shape; AB_LOGITS=1 times the logits form."""
 import ctypes, os, sys
 import torch
 
-K, B, X = 50, int(os.environ.get("AB_B", 1024)), 784
+K, B, X = int(os.environ.get("AB_K", 50)), int(os.environ.get("AB_B", 1024)), 784
+LOGITS = os.environ.get("AB_LOGITS", "0") == "1"
 c = ctypes
 vp, i64, i32, dbl = c.c_void_p, c.c_int64, c.c_int, c.c_double
 libs = []
@@ -26,7 +28,9 @@ for arg in sys.argv[1:]:
     libs.append((name, lib))
 dev = "cuda"
 torch.manual_seed(0)
-probs = torch.sigmoid(2 * torch.randn(K, B, X, device=dev))
+probs = 2 * torch.randn(K, B, X, device=dev)
+if not LOGITS:
+    probs = torch.sigmoid(probs)
 x = (torch.rand(B, X, device=dev) < 0.5).float()
 other = torch.randn(K, B, device=dev) - 55
 logq = torch.randn(K, B, device=dev) + 30
@@ -57,7 +61,7 @@ def first_call(name, lib):
 def run(lib, o, est):
     rc = lib.zs_iw_bernoulli_fused(est, o["cost"].data_ptr(), o["dprobs"].data_ptr(), o["dlogp"].data_ptr(),
                                    o["dlogq"].data_ptr(), None, probs.data_ptr(), x.data_ptr(), other.data_ptr(),
-                                   logq.data_ptr(), K, B, X, 1.0 / B, 0, stream)
+                                   logq.data_ptr(), K, B, X, 1.0 / B, 2 if LOGITS else 0, stream)  # ZS_FUSED_LOGITS = 2
     assert rc == 0, rc
 
 

@@ -678,6 +678,16 @@ __device__ __forceinline__ void tma_load_box(void* dst_smem, const CUtensorMap* 
         : "memory");
 }
 
+// tma_load_box with an L2 cache policy (createpolicy), e.g. evict-first for data that is read exactly once
+__device__ __forceinline__ void tma_load_box_hint(void* dst_smem, const CUtensorMap* map, int c0, int c1, int c2,
+                                                  uint64_t* bar, uint64_t policy) {
+    asm volatile(
+        "cp.async.bulk.tensor.3d.shared::cluster.global.tile.mbarrier::complete_tx::bytes.L2::cache_hint [%0], [%1, {%2, %3, %4}], [%5], %6;" ::"r"(
+            smem_u32(dst_smem)),
+        "l"(map), "r"(c0), "r"(c1), "r"(c2), "r"(smem_u32(bar)), "l"(policy)
+        : "memory");
+}
+
 // request a box into L2 only (no shared-memory destination, no completion tracking)
 __device__ __forceinline__ void tma_prefetch_box_l2(const CUtensorMap* map, int c0, int c1, int c2) {
     asm volatile("cp.async.bulk.prefetch.tensor.3d.L2.global.tile [%0, {%1, %2, %3}];" ::"l"(map), "r"(c0), "r"(c1), "r"(c2)
@@ -1281,8 +1291,12 @@ __global__ void __launch_bounds__((BOX_MAX_ROW_WARPS + 4) * 32, 1)
     __syncthreads();
 
     if (is_producer) {
-        // box t = (column t / NBOX, piece t % NBOX) goes to slot t % nslot
+        // box t = (column t / NBOX, piece t % NBOX) goes to slot t % nslot.  probs is read exactly once: its lines
+        // are marked evict-first, so that 160 MB of it does not push out of L2 what the launch writes and the
+        // kernels around it read.  Measured on one B200: the IWAE step 83.1 -> 78.9 us (profiles/r3_boxf_rows.md)
         if (lane == 0) {
+            uint64_t evict_first;
+            asm volatile("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(evict_first));
             int slot = 0, q = 0;
             uint32_t wait_parity = 1;
             bool first_pass = true;
@@ -1291,7 +1305,8 @@ __global__ void __launch_bounds__((BOX_MAX_ROW_WARPS + 4) * 32, 1)
             for (int64_t t = 0; t < ntask; ++t) {
                 if (!first_pass) mbar_wait(&empty[slot], wait_parity);
                 mbar_expect_tx(&full[slot], box_bytes);
-                tma_load_box(slots + (size_t)slot * slot_bytes, &probs_map, q * INNER, (int)col, 0, &full[slot]);
+                tma_load_box_hint(slots + (size_t)slot * slot_bytes, &probs_map, q * INNER, (int)col, 0, &full[slot],
+                                  evict_first);
                 if (++q == NBOX) { q = 0; col += gridDim.x; }
                 if (++slot == nslot) {
                     slot = 0;
@@ -1740,8 +1755,12 @@ int launch_fused_box(const FusedCall& c, bool generic_only) {
 #undef ZS_BOXF_PICK
     }
     if (fixed != nullptr) {
+        // Bernoulli at K <= 25: two rows per row warp as well, not one row per warp (whose row b repeats row a and is
+        // dropped): the warp's x load serves two rows.  Measured on one B200 at K = 25, B = 1024, X = 784:
+        // 47.7 -> 37.7 us (profiles/r3_boxf_rows.md)
+        const int nw_fixed = c.poisson ? nw : (int)((K + 1) / 2);
         ZS_CUDA_TRY(cudaFuncSetAttribute(fixed, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        launch_pdl(PDL_FUSED, fixed, dim3((unsigned)grid), dim3(threads), smem, c.st, map, c.cost, c.dprobs, c.dlogp, c.dlogq,
+        launch_pdl(PDL_FUSED, fixed, dim3((unsigned)grid), dim3((nw_fixed + 4) * 32), smem, c.st, map, c.cost, c.dprobs, c.dlogp, c.dlogq,
                    c.logpx_out, c.x, c.logp_other, c.logq, (int)K, B, nslot, (float)c.grad_scale, stg.groups, stg.cycles,
                    c.kflags, c.ldkb, c.loss_out, c.ticket);
         ZS_LAUNCH_CHECK(c.poisson ? "k_iw_poisson_boxf" : "k_iw_bernoulli_boxf");
