@@ -292,6 +292,81 @@ def categorical_sample(logits, u, K, M, C):
     return out.reshape(K, M)
 
 
+# --------------------------------------------------------------------------- Poisson (explicit operand modes)
+def poisson_sample(rate, mode, K, N, seed, offset):
+    """rate: numpy array laid out for `mode` (FULL [K*N], KBCAST [N], SCALAR [1]) -> [K, N] counts."""
+    dt = rate.dtype.type
+    rate = _c(rate, dt)
+    out = np.empty(K * N, dt)
+    _call("orc_poisson_sample", dt, _p(out), _p(rate), mode, _i64(K), _i64(N), ctypes.c_uint64(seed),
+          ctypes.c_uint64(offset))
+    return out.reshape(K, N)
+
+
+def poisson_logpmf_fwd(x, xm, rate, rm, K, M, E):
+    dt = rate.dtype.type
+    x, rate = _c(x, dt), _c(rate, dt)
+    out = np.empty(K * M, dt)
+    _call("orc_poisson_logpmf_fwd", dt, _p(out), _p(x), xm, _p(rate), rm, _i64(K), _i64(M), _i64(E))
+    return out.reshape(K, M)
+
+
+def poisson_logpmf_bwd(g, x, xm, rate, rm, K, M, E):
+    dt = rate.dtype.type
+    g, x, rate = _c(g, dt), _c(x, dt), _c(rate, dt)
+    drate = np.empty(rate.size, dt)
+    _call("orc_poisson_logpmf_bwd", dt, _p(drate), _p(g), _p(x), xm, _p(rate), rm, _i64(K), _i64(M), _i64(E))
+    return drate.reshape(rate.shape)
+
+
+def iw_poisson_step(estimator, rate, x, logp_other, logq, grad_scale, need_drate=True):
+    """The fused Poisson step restated: log-pmf -> IW objective -> rate gradient.
+    rate [K,B,X], x [B,X], logp_other/logq [K,B] or None.  Returns dict(cost, drate, dlogp, dlogq, logpx)."""
+    K, B, X = rate.shape
+    lpx = poisson_logpmf_fwd(x, KBCAST, rate, FULL, K, B, X)
+    lp = lpx if logp_other is None else lpx + logp_other
+    lq = np.zeros_like(lpx) if logq is None else logq
+    cost, dlp, dlq = iw_objective(estimator, lp, lq, grad_scale)
+    drate = poisson_logpmf_bwd(dlp, x, KBCAST, rate, FULL, K, B, X) if need_drate else None
+    return dict(cost=cost, drate=drate, dlogp=dlp, dlogq=dlq, logpx=lpx)
+
+
+# --------------------------------------------------------------------------- Beta (explicit operand modes)
+def digamma(x, dtype=np.float64):
+    """psi as the Beta gradients evaluate it, elementwise in `dtype`."""
+    f = getattr(lib(), "orc_digamma" + _sfx(dtype))
+    f.restype, f.argtypes = ctypes.c_double, [ctypes.c_double]
+    return np.array([f(float(v)) for v in np.ravel(x)], dtype).reshape(np.shape(x))
+
+
+def beta_sample(alpha, am, beta, bm, K, N, seed, offset):
+    """alpha / beta: numpy arrays laid out for their modes (FULL [K*N], KBCAST [N], SCALAR [1]) -> [K, N] samples."""
+    dt = alpha.dtype.type
+    alpha, beta = _c(alpha, dt), _c(beta, dt)
+    out = np.empty(K * N, dt)
+    _call("orc_beta_sample", dt, _p(out), _p(alpha), am, _p(beta), bm, _i64(K), _i64(N), ctypes.c_uint64(seed),
+          ctypes.c_uint64(offset))
+    return out.reshape(K, N)
+
+
+def beta_logprob_fwd(x, xm, a, am, b, bm, K, M, E):
+    dt = a.dtype.type
+    x, a, b = _c(x, dt), _c(a, dt), _c(b, dt)
+    out = np.empty(K * M, dt)
+    _call("orc_beta_logprob_fwd", dt, _p(out), _p(x), xm, _p(a), am, _p(b), bm, _i64(K), _i64(M), _i64(E))
+    return out.reshape(K, M)
+
+
+def beta_logprob_bwd(g, x, xm, a, am, b, bm, K, M, E, need=(True, True, True)):
+    """(dx, da, db), each with the layout of its operand (None where not needed)."""
+    dt = a.dtype.type
+    g, x, a, b = _c(g, dt), _c(x, dt), _c(a, dt), _c(b, dt)
+    outs = [np.empty(v.size, dt) if n else None for v, n in zip((x, a, b), need)]
+    _call("orc_beta_logprob_bwd", dt, *[_p(o) for o in outs], _p(g), _p(x), xm, _p(a), am, _p(b), bm, _i64(K),
+          _i64(M), _i64(E))
+    return tuple(None if o is None else o.reshape(v.shape) for o, v in zip(outs, (x, a, b)))
+
+
 # --------------------------------------------------------------------------- objectives
 def log_mean_exp(x):
     """axis-0 log_mean_exp of [K,B] (zhusuan/utils.py:6-21)."""

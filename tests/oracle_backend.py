@@ -130,7 +130,23 @@ def bernoulli_logpmf_bwd(g, x, xm, probs, pm, K, M, E, need_x, need_probs, logit
     return (_t(dx, probs) if need_x else None, _t(dp, probs) if need_probs else None)
 
 
-FAM_LOGISTIC, FAM_LAPLACE = 1, 2
+def poisson_sample(rate, rm, K, N, seed=0, offset=0, rng_state=None):
+    return _t(O.poisson_sample(_np(rate), rm, K, N, seed, offset), rate)
+
+
+def poisson_logpmf_fwd(x, xm, rate, rm, K, M, E):
+    return _t(O.poisson_logpmf_fwd(_np(x), xm, _np(rate), rm, K, M, E), rate)
+
+
+def poisson_logpmf_bwd(g, x, xm, rate, rm, K, M, E):
+    return _t(O.poisson_logpmf_bwd(_np(g), _np(x), xm, _np(rate), rm, K, M, E), rate)
+
+
+def beta_sample(alpha, am, beta, bm, K, N, seed=0, offset=0, rng_state=None):
+    return _t(O.beta_sample(_np(alpha), am, _np(beta), bm, K, N, seed, offset), alpha)
+
+
+FAM_LOGISTIC, FAM_LAPLACE, FAM_BETA = 1, 2, 4
 
 
 def _locscale_u(family, K, N, dtype, u_in, seed, offset):
@@ -155,10 +171,16 @@ def locscale_sample_bwd(family, dz, loc_like, loc_mode, scale_like, scale_mode, 
 
 
 def locscale_logprob_fwd(family, x, xm, loc, lm, scale, sm, K, M, E):
+    if family == FAM_BETA:  # loc = alpha, scale = beta
+        return _t(O.beta_logprob_fwd(_np(x), xm, _np(loc), lm, _np(scale), sm, K, M, E), x)
     return _t(O.locscale_logprob_fwd(family, _np(x), _np(loc), _np(scale), K, M, E), x)
 
 
 def locscale_logprob_bwd(family, g, x, xm, loc, lm, scale, sm, K, M, E, need_x, need_loc, need_scale):
+    if family == FAM_BETA:
+        outs = O.beta_logprob_bwd(_np(g), _np(x), xm, _np(loc), lm, _np(scale), sm, K, M, E,
+                                  need=(need_x, need_loc, need_scale))
+        return tuple(None if o is None else _t(o, x) for o in outs)
     dx, dl, ds = O.locscale_logprob_bwd(family, _np(g), _np(x), _np(loc), _np(scale), K, M, E)
     return (_t(dx.reshape(x.shape), x) if need_x else None, _t(dl.reshape(loc.shape), x) if need_loc else None,
             _t(ds.reshape(scale.shape), x) if need_scale else None)
@@ -216,6 +238,15 @@ def iw_bernoulli_fused(estimator, probs, x, logp_other, logq, grad_scale, need_d
     return dict(cost=_t(cost, probs), dprobs=_t(r["dprobs"], probs) if need_dprobs else None,
                 dlogp=_t(r["dlogp"], probs), dlogq=_t(r["dlogq"], probs),
                 logpx=_t(r["logpx"], probs) if want_logpx else None)
+
+
+def iw_poisson_fused(estimator, rate, x, logp_other, logq, grad_scale, need_drate=True, want_logpx=False, out=None,
+                     accumulate_cost=False, cost_scaled=False, want_loss=False):
+    r = O.iw_poisson_step(estimator, _np(rate), _np(x), _np(logp_other), _np(logq), grad_scale, need_drate)
+    cost = r["cost"] * (np.float32(grad_scale) if cost_scaled else np.float32(1.0))
+    return dict(cost=_t(cost, rate), dprobs=_t(r["drate"], rate) if need_drate else None,
+                dlogp=_t(r["dlogp"], rate), dlogq=_t(r["dlogq"], rate),
+                logpx=_t(r["logpx"], rate) if want_logpx else None)
 
 
 def reinforce_step(logp, logq, moving_mean, local_step, decay, need_grads=True):
@@ -335,10 +366,11 @@ def install(monkeypatch):
     from zhusuan import _backend, _ops, _rng
     for name in ("normal_sample", "normal_sample_bwd", "normal_logprob_fwd", "normal_logprob_bwd", "normal_latent_fwd", "normal_latent_bwd",
                  "bernoulli_latent_fwd", "bernoulli_latent_bwd", "bernoulli_sample",
-                 "bernoulli_logpmf_fwd", "bernoulli_logpmf_bwd", "locscale_sample", "locscale_sample_bwd",
+                 "bernoulli_logpmf_fwd", "bernoulli_logpmf_bwd", "poisson_sample", "poisson_logpmf_fwd",
+                 "poisson_logpmf_bwd", "beta_sample", "locscale_sample", "locscale_sample_bwd",
                  "locscale_logprob_fwd", "locscale_logprob_bwd", "categorical_sample", "categorical_logpmf_fwd",
                  "categorical_logpmf_bwd", "iw_objective", "combine_sums", "log_mean_exp", "log_mean_exp_bwd", "fused_supported",
-                 "iw_bernoulli_fused", "reinforce_step", "scale_inplace", "philox_normal", "sgld_step", "psgld_step", "sghmc_pre",
+                 "iw_bernoulli_fused", "iw_poisson_fused", "reinforce_step", "scale_inplace", "philox_normal", "sgld_step", "psgld_step", "sghmc_pre",
                  "sghmc_post", "sgmcmc_multi_step"):
         monkeypatch.setattr(_backend, name, globals()[name])
     monkeypatch.setattr(_backend, "require_cuda", lambda: None)

@@ -3,7 +3,7 @@ StochasticTensor reductions, every row-kernel path), the sampler, BayesianNet re
 under the two estimators for non-reparameterised latents.
 
 Modes as in tests/test_poisson.py: `oracle` (CPU; the ctypes backend replaced by the CPU oracle, with the Beta node
-restated in tests/beta_oracle.c), `cuda` (B200 kernels, CUDA tensors) and `cuda-host` (CPU tensors in and out).
+restated in oracle/zs_oracle_impl.h), `cuda` (B200 kernels, CUDA tensors) and `cuda-host` (CPU tensors in and out).
 The anchor is torch.distributions.Beta in float64, the function the reference's Beta delegates to, cross-checked with
 scipy.  Parity rule (DESIGN.md §4): float64 within 1e-12 normwise; float32 within 1e-5 normwise of float64 torch, or
 no farther from it than float32 torch is.  Non-finite entries must match float64 torch exactly.
@@ -31,8 +31,9 @@ FULL, KBCAST, SCALAR = _backend.FULL, _backend.KBCAST, _backend.SCALAR
 def dev(request, monkeypatch):
     mode = request.param
     if mode == "oracle":
-        import beta_oracle
-        beta_oracle.install(monkeypatch)
+        import oracle_backend
+        request.getfixturevalue("oracle")  # rebuilds the oracle library if its sources changed
+        oracle_backend.install(monkeypatch)
         return torch.device("cpu")
     return torch.device("cuda") if mode == "cuda" else torch.device("cpu")
 
@@ -345,8 +346,7 @@ DISAGREE_MAX = 1e-3
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("dtype", [torch.float32, torch.float64])
-def test_sampler_matches_oracle_geometry_and_modes(dtype):
-    import beta_oracle
+def test_sampler_matches_oracle_geometry_and_modes(oracle, dtype):
     rng = np.random.RandomState(35)
     n = 200000
     a = np.exp(rng.uniform(-4, 6, n)).astype(_np_dtype(dtype))
@@ -356,7 +356,7 @@ def test_sampler_matches_oracle_geometry_and_modes(dtype):
     small = _backend.beta_sample(ta[:1000].contiguous(), FULL, tb[:1000].contiguous(), FULL, 1, 1000, seed=91,
                                  offset=8)
     assert torch.equal(big[0, :1000], small[0])  # a 1000-element launch draws what a 200000-element launch drew
-    ref = beta_oracle.beta_sample(a, FULL, b, FULL, 1, n, 91, 8)
+    ref = oracle.beta_sample(a, FULL, b, FULL, 1, n, 91, 8)
     assert np.mean(~np.isclose(big.cpu().numpy(), ref, rtol=1e-6, atol=0)) <= DISAGREE_MAX
     # KBCAST and SCALAR parameters draw what the same values expanded to FULL draw
     K, N = 4, 500
@@ -364,7 +364,7 @@ def test_sampler_matches_oracle_geometry_and_modes(dtype):
     full = _backend.beta_sample(ta[:N].repeat(K).contiguous(), FULL, tb[:N].repeat(K).contiguous(), FULL, K, N,
                                 seed=91, offset=8)
     assert torch.equal(kb, full)
-    ref_kb = beta_oracle.beta_sample(a[:N], KBCAST, b[:N], KBCAST, K, N, 91, 8)
+    ref_kb = oracle.beta_sample(a[:N], KBCAST, b[:N], KBCAST, K, N, 91, 8)
     assert np.mean(~np.isclose(kb.cpu().numpy(), ref_kb, rtol=1e-6, atol=0)) <= DISAGREE_MAX
     sc = _backend.beta_sample(ta[:1].contiguous(), SCALAR, tb[:1].contiguous(), SCALAR, K, N, seed=91, offset=8)
     sc_full = _backend.beta_sample(ta[:1].expand(K * N).contiguous(), FULL, tb[:1].expand(K * N).contiguous(), FULL,

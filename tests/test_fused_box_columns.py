@@ -6,7 +6,7 @@ from the wrong column only shows once a CTA takes >= 4 columns, so B = 4 G + 3 h
 takes at least 4 columns and the grid does not divide B.  Neighbouring columns differ strongly (counts, binary or
 fractional x, logp_other, logq), so a wrong slot moves log p(x | z) or the cost by tens of nats.
 
-References: oracle.iw_bernoulli_step, oracle.iw_bernoulli_logits_step and tests/poisson_oracle.iw_poisson_step in
+References: oracle.iw_bernoulli_step, oracle.iw_bernoulli_logits_step and oracle.iw_poisson_step in
 float64 for log p(x | z) and the cost; the gradients staged as in test_gpu_kernels.test_fused_vs_oracle (the oracle
 fed the kernel's own log p(x | z), since the weights see exp() of float32 log-weights).  Every comparison is
 elementwise, with the scale of the element's own column or row.
@@ -67,20 +67,18 @@ def _np(t):
 
 
 def _oracle_step(oracle, form, est, p, x, other, logq):
-    import poisson_oracle
     code = oracle.SGVB if est == be.SGVB else oracle.VIMCO
     args = (code, _np(p), _np(x), _np(other), _np(logq))
     if form == "poisson":
-        return poisson_oracle.iw_poisson_step(*args, 1.0 / x.shape[0], need_drate=False)
+        return oracle.iw_poisson_step(*args, 1.0 / x.shape[0], need_drate=False)
     step = oracle.iw_bernoulli_logits_step if form == "logits" else oracle.iw_bernoulli_step
     return step(*args, need_dprobs=False)
 
 
 def _oracle_bwd(oracle, form, g, p, x):
-    import poisson_oracle
     K, B, X = p.shape
     if form == "poisson":
-        return poisson_oracle.poisson_logpmf_bwd(g, _np(x), 1, _np(p), 0, K, B, X)
+        return oracle.poisson_logpmf_bwd(g, _np(x), oracle.KBCAST, _np(p), oracle.FULL, K, B, X)
     if form == "logits":
         return oracle.bernoulli_logits_logpmf_bwd(g, _np(x), _np(p), K, B, X)
     return oracle.bernoulli_logpmf_bwd(g, _np(x), _np(p), K, B, X)

@@ -2,7 +2,7 @@
 the sampler, BayesianNet registration and the fused Poisson-likelihood importance-weighted step.
 
 Modes as in tests/test_api.py: `oracle` (CPU; the ctypes backend replaced by the CPU oracle, with the Poisson node
-restated in tests/poisson_oracle.c), `cuda` (B200 kernels, CUDA tensors) and `cuda-host` (CPU tensors in and out).
+restated in oracle/zs_oracle_impl.h), `cuda` (B200 kernels, CUDA tensors) and `cuda-host` (CPU tensors in and out).
 The anchor is torch.distributions.Poisson, the function the reference's Poisson delegates to, cross-checked with scipy.
 Parity rule (DESIGN.md §4): within 1e-5 normwise of float32 torch, or no farther from float64 torch than float32 torch is.
 """
@@ -28,8 +28,9 @@ MODES = [pytest.param("oracle"), pytest.param("cuda", marks=pytest.mark.gpu),
 def dev(request, monkeypatch):
     mode = request.param
     if mode == "oracle":
-        import poisson_oracle
-        poisson_oracle.install(monkeypatch)
+        import oracle_backend
+        request.getfixturevalue("oracle")  # rebuilds the oracle library if its sources changed
+        oracle_backend.install(monkeypatch)
         return torch.device("cpu")
     return torch.device("cuda") if mode == "cuda" else torch.device("cpu")
 
@@ -236,8 +237,7 @@ DISAGREE_MAX = 1e-3
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("dtype", [torch.float32, torch.float64])
-def test_sampler_matches_oracle_and_geometry(dtype):
-    import poisson_oracle
+def test_sampler_matches_oracle_and_geometry(oracle, dtype):
     rng = np.random.RandomState(14)
     n = 200000
     rate = np.concatenate([rng.uniform(0, 10, n // 2), rng.uniform(10, 500, n // 2)])
@@ -246,8 +246,8 @@ def test_sampler_matches_oracle_and_geometry(dtype):
     small = _backend.poisson_sample(r[:1000].contiguous(), _backend.FULL, 1, 1000, seed=77, offset=8)
     assert torch.equal(big[0, :1000], small[0])  # a 1000-element grid draws what a 200000-element grid drew
     kb = _backend.poisson_sample(r[:500].contiguous(), _backend.KBCAST, 4, 500, seed=77, offset=8)
-    ref_kb = poisson_oracle.poisson_sample(rate[:500].astype(_np_dtype(dtype)), _backend.KBCAST, 4, 500, 77, 8)
-    ref = poisson_oracle.poisson_sample(rate.astype(_np_dtype(dtype)), _backend.FULL, 1, n, 77, 8)
+    ref_kb = oracle.poisson_sample(rate[:500].astype(_np_dtype(dtype)), _backend.KBCAST, 4, 500, 77, 8)
+    ref = oracle.poisson_sample(rate.astype(_np_dtype(dtype)), _backend.FULL, 1, n, 77, 8)
     assert np.mean(big.cpu().numpy() != ref) <= DISAGREE_MAX
     assert np.mean(kb.cpu().numpy() != ref_kb) <= DISAGREE_MAX
     other = _backend.poisson_sample(r, _backend.FULL, 1, n, seed=77, offset=12)  # the next stream position
@@ -410,10 +410,9 @@ def test_fused_kernel_dispatch_and_fallback():
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("est", [_backend.SGVB, _backend.VIMCO])
-def test_fused_kernel_entry_point_against_restatement(est):
+def test_fused_kernel_entry_point_against_restatement(oracle, est):
     """zs_iw_poisson_fused at each instantiated row length (K = 50 and K = 7), against the oracle restatement; with
     counts that are mostly zero and rates of at least 0.01 (zero and subnormal rates: tests/test_fused_box_columns.py)."""
-    import poisson_oracle
     rng = np.random.RandomState(24)
     for X, K in ((128, 50), (256, 7), (512, 50), (784, 50), (1024, 33)):
         B = 5
@@ -423,8 +422,8 @@ def test_fused_kernel_entry_point_against_restatement(est):
         lq = rng.standard_normal((K, B)).astype(np.float32)
         t = lambda a: torch.tensor(a, device="cuda")
         r = _backend.iw_poisson_fused(est, t(rate), t(x), t(lo), t(lq), 1.0 / B, want_logpx=True)
-        ref = poisson_oracle.iw_poisson_step(est, rate.astype(np.float64), x.astype(np.float64), lo.astype(np.float64),
-                                             lq.astype(np.float64), 1.0 / B)
+        ref = oracle.iw_poisson_step(est, rate.astype(np.float64), x.astype(np.float64), lo.astype(np.float64),
+                                     lq.astype(np.float64), 1.0 / B)
         assert _normwise(r["logpx"], ref["logpx"]) < 1e-6, X
         assert _normwise(r["cost"], ref["cost"]) < 2e-5, X
         assert _normwise(r["dlogp"], ref["dlogp"]) < 2e-5, X
