@@ -155,18 +155,10 @@ __global__ void __launch_bounds__(256) k_cat_sample(T* __restrict__ out, const T
 using namespace zs;
 
 #define ZS_CAT_SWITCH(dtype, C, ...)                                  \
-    if ((dtype) == ZS_F32) {                                          \
-        using T = float;                                              \
+    ZS_DTYPE_SWITCH(dtype, {                                          \
         if ((C) <= 16) { constexpr int LPR = 4; __VA_ARGS__ }         \
         else { constexpr int LPR = 32; __VA_ARGS__ }                  \
-    } else if ((dtype) == ZS_F64) {                                   \
-        using T = double;                                             \
-        if ((C) <= 16) { constexpr int LPR = 4; __VA_ARGS__ }         \
-        else { constexpr int LPR = 32; __VA_ARGS__ }                  \
-    } else {                                                          \
-        set_last_error_msg("dtype must be ZS_F32 or ZS_F64");         \
-        return ZS_ERR_DTYPE;                                          \
-    }
+    })
 
 extern "C" {
 
@@ -177,16 +169,10 @@ int zs_categorical_sample(int dtype, void* out, const void* logits, int logits_m
     ZS_REQUIRE(logits_mode == ZS_FULL || logits_mode == ZS_KBCAST, ZS_ERR_ARG);
     if (K * M == 0) return ZS_OK;
     const int grid = grid_for(K * M, 256);
-    if (dtype == ZS_F32)
-        k_cat_sample<float><<<grid, 256, 0, as_stream(stream)>>>((float*)out, (const float*)logits, logits_mode,
-                                                                  (const float*)u_in, K, M, C, seed, offset, rs);
-    else if (dtype == ZS_F64)
-        k_cat_sample<double><<<grid, 256, 0, as_stream(stream)>>>((double*)out, (const double*)logits, logits_mode,
-                                                                   (const double*)u_in, K, M, C, seed, offset, rs);
-    else {
-        set_last_error_msg("dtype must be ZS_F32 or ZS_F64");
-        return ZS_ERR_DTYPE;
-    }
+    ZS_DTYPE_SWITCH(dtype, {
+        k_cat_sample<T><<<grid, 256, 0, as_stream(stream)>>>((T*)out, (const T*)logits, logits_mode, (const T*)u_in, K,
+                                                              M, C, seed, offset, rs);
+    })
     ZS_LAUNCH_CHECK("k_cat_sample");
     return ZS_OK;
 }

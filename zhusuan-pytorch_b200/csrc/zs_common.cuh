@@ -38,6 +38,20 @@ void set_last_error_msg(const char* msg);
         }                                                  \
     } while (0)
 
+// Runs the statements with `T` bound to the element type of `dtype`; any other dtype returns ZS_ERR_DTYPE from the
+// enclosing entry point.
+#define ZS_DTYPE_SWITCH(dtype, ...)                                      \
+    if ((dtype) == ZS_F32) {                                             \
+        using T = float;                                                 \
+        __VA_ARGS__                                                      \
+    } else if ((dtype) == ZS_F64) {                                      \
+        using T = double;                                                \
+        __VA_ARGS__                                                      \
+    } else {                                                             \
+        ::zs::set_last_error_msg("dtype must be ZS_F32 or ZS_F64");      \
+        return ZS_ERR_DTYPE;                                             \
+    }
+
 inline bool valid_mode(int m) { return m == ZS_FULL || m == ZS_KBCAST || m == ZS_SCALAR; }
 inline bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }
 inline cudaStream_t as_stream(zs_stream_t s) { return reinterpret_cast<cudaStream_t>(s); }

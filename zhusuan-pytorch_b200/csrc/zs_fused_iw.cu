@@ -1845,6 +1845,31 @@ int fused_launch(const FusedCall& c) {
     return launch_fused_ring(c);
 }
 
+// The checks and the FusedCall of the four fused entry points.  `with_loss`: the _loss form, which also writes the
+// mean objective and so needs loss_out, workspace, cost, at least one column and a grid its workspace covers.
+int fused_entry(bool poisson, bool with_loss, int estimator, float* loss_out, void* workspace, float* cost,
+                float* dprobs, float* dlogp, float* dlogq, float* logpx_out, const float* probs, const float* x,
+                const float* logp_other, const float* logq, int64_t K, int64_t B, int64_t X, double grad_scale,
+                int flags, zs_stream_t stream) {
+    ZS_REQUIRE(probs && x && K >= 1 && B >= 0 && X >= 1, ZS_ERR_ARG);
+    ZS_REQUIRE(!with_loss || (loss_out && workspace && cost && B >= 1), ZS_ERR_ARG);
+    ZS_REQUIRE(estimator == ZS_EST_SGVB || estimator == ZS_EST_VIMCO, ZS_ERR_ARG);
+    ZS_REQUIRE(!(estimator == ZS_EST_VIMCO && (K < 2 || logq == nullptr)), ZS_ERR_ARG);
+    const int allowed = ZS_FUSED_ACCUMULATE_COST | ZS_FUSED_COST_SCALED | (poisson ? 0 : ZS_FUSED_LOGITS);
+    ZS_REQUIRE((flags & ~allowed) == 0, ZS_ERR_ARG);
+    if (B == 0) return ZS_OK;
+    if (with_loss) ZS_REQUIRE(persistent_grid(B) <= ZS_FUSED_LOSS_MAX_GRID, ZS_ERR_UNSUPPORTED);
+    FusedCall c{estimator, cost, dprobs, dlogp, dlogq, logpx_out, probs, x, logp_other, logq, K, B, X, B, grad_scale,
+                ((flags & ZS_FUSED_ACCUMULATE_COST) ? FUSED_ACCUMULATE : 0) |
+                    ((flags & ZS_FUSED_COST_SCALED) ? FUSED_COST_SCALED : 0),
+                (flags & ZS_FUSED_LOGITS) != 0,
+                as_stream(stream),
+                loss_out,
+                (unsigned*)workspace,
+                poisson};
+    return fused_launch(c);
+}
+
 }  // namespace
 
 extern "C" {
@@ -1852,71 +1877,31 @@ extern "C" {
 int zs_iw_bernoulli_fused(int estimator, float* cost, float* dprobs, float* dlogp, float* dlogq, float* logpx_out,
                           const float* probs, const float* x, const float* logp_other, const float* logq, int64_t K,
                           int64_t B, int64_t X, double grad_scale, int flags, zs_stream_t stream) {
-    ZS_REQUIRE(probs && x && K >= 1 && B >= 0 && X >= 1, ZS_ERR_ARG);
-    ZS_REQUIRE(estimator == ZS_EST_SGVB || estimator == ZS_EST_VIMCO, ZS_ERR_ARG);
-    ZS_REQUIRE(!(estimator == ZS_EST_VIMCO && (K < 2 || logq == nullptr)), ZS_ERR_ARG);
-    ZS_REQUIRE((flags & ~(ZS_FUSED_ACCUMULATE_COST | ZS_FUSED_LOGITS | ZS_FUSED_COST_SCALED)) == 0, ZS_ERR_ARG);
-    if (B == 0) return ZS_OK;
-    FusedCall c{estimator, cost, dprobs, dlogp, dlogq, logpx_out, probs, x, logp_other, logq, K, B, X, B, grad_scale,
-                ((flags & ZS_FUSED_ACCUMULATE_COST) ? FUSED_ACCUMULATE : 0) |
-                    ((flags & ZS_FUSED_COST_SCALED) ? FUSED_COST_SCALED : 0),
-                (flags & ZS_FUSED_LOGITS) != 0,
-                as_stream(stream)};
-    return fused_launch(c);
+    return fused_entry(false, false, estimator, nullptr, nullptr, cost, dprobs, dlogp, dlogq, logpx_out, probs, x,
+                       logp_other, logq, K, B, X, grad_scale, flags, stream);
 }
 
 int zs_iw_bernoulli_fused_loss(int estimator, float* loss_out, void* workspace, float* cost, float* dprobs, float* dlogp,
                                float* dlogq, float* logpx_out, const float* probs, const float* x,
                                const float* logp_other, const float* logq, int64_t K, int64_t B, int64_t X,
                                double grad_scale, int flags, zs_stream_t stream) {
-    ZS_REQUIRE(probs && x && loss_out && workspace && cost && K >= 1 && B >= 1 && X >= 1, ZS_ERR_ARG);
-    ZS_REQUIRE(estimator == ZS_EST_SGVB || estimator == ZS_EST_VIMCO, ZS_ERR_ARG);
-    ZS_REQUIRE(!(estimator == ZS_EST_VIMCO && (K < 2 || logq == nullptr)), ZS_ERR_ARG);
-    ZS_REQUIRE((flags & ~(ZS_FUSED_ACCUMULATE_COST | ZS_FUSED_LOGITS | ZS_FUSED_COST_SCALED)) == 0, ZS_ERR_ARG);
-    FusedCall c{estimator, cost, dprobs, dlogp, dlogq, logpx_out, probs, x, logp_other, logq, K, B, X, B, grad_scale,
-                ((flags & ZS_FUSED_ACCUMULATE_COST) ? FUSED_ACCUMULATE : 0) |
-                    ((flags & ZS_FUSED_COST_SCALED) ? FUSED_COST_SCALED : 0),
-                (flags & ZS_FUSED_LOGITS) != 0,
-                as_stream(stream)};
-    ZS_REQUIRE(persistent_grid(B) <= ZS_FUSED_LOSS_MAX_GRID, ZS_ERR_UNSUPPORTED);
-    c.loss_out = loss_out;
-    c.ticket = (unsigned*)workspace;
-    return fused_launch(c);
+    return fused_entry(false, true, estimator, loss_out, workspace, cost, dprobs, dlogp, dlogq, logpx_out, probs, x,
+                       logp_other, logq, K, B, X, grad_scale, flags, stream);
 }
 
 int zs_iw_poisson_fused(int estimator, float* cost, float* drate, float* dlogp, float* dlogq, float* logpx_out,
                         const float* rate, const float* x, const float* logp_other, const float* logq, int64_t K,
                         int64_t B, int64_t X, double grad_scale, int flags, zs_stream_t stream) {
-    ZS_REQUIRE(rate && x && K >= 1 && B >= 0 && X >= 1, ZS_ERR_ARG);
-    ZS_REQUIRE(estimator == ZS_EST_SGVB || estimator == ZS_EST_VIMCO, ZS_ERR_ARG);
-    ZS_REQUIRE(!(estimator == ZS_EST_VIMCO && (K < 2 || logq == nullptr)), ZS_ERR_ARG);
-    ZS_REQUIRE((flags & ~(ZS_FUSED_ACCUMULATE_COST | ZS_FUSED_COST_SCALED)) == 0, ZS_ERR_ARG);
-    if (B == 0) return ZS_OK;
-    FusedCall c{estimator, cost, drate, dlogp, dlogq, logpx_out, rate, x, logp_other, logq, K, B, X, B, grad_scale,
-                ((flags & ZS_FUSED_ACCUMULATE_COST) ? FUSED_ACCUMULATE : 0) |
-                    ((flags & ZS_FUSED_COST_SCALED) ? FUSED_COST_SCALED : 0),
-                false, as_stream(stream)};
-    c.poisson = true;
-    return fused_launch(c);
+    return fused_entry(true, false, estimator, nullptr, nullptr, cost, drate, dlogp, dlogq, logpx_out, rate, x,
+                       logp_other, logq, K, B, X, grad_scale, flags, stream);
 }
 
 int zs_iw_poisson_fused_loss(int estimator, float* loss_out, void* workspace, float* cost, float* drate, float* dlogp,
                              float* dlogq, float* logpx_out, const float* rate, const float* x, const float* logp_other,
                              const float* logq, int64_t K, int64_t B, int64_t X, double grad_scale, int flags,
                              zs_stream_t stream) {
-    ZS_REQUIRE(rate && x && loss_out && workspace && cost && K >= 1 && B >= 1 && X >= 1, ZS_ERR_ARG);
-    ZS_REQUIRE(estimator == ZS_EST_SGVB || estimator == ZS_EST_VIMCO, ZS_ERR_ARG);
-    ZS_REQUIRE(!(estimator == ZS_EST_VIMCO && (K < 2 || logq == nullptr)), ZS_ERR_ARG);
-    ZS_REQUIRE((flags & ~(ZS_FUSED_ACCUMULATE_COST | ZS_FUSED_COST_SCALED)) == 0, ZS_ERR_ARG);
-    FusedCall c{estimator, cost, drate, dlogp, dlogq, logpx_out, rate, x, logp_other, logq, K, B, X, B, grad_scale,
-                ((flags & ZS_FUSED_ACCUMULATE_COST) ? FUSED_ACCUMULATE : 0) |
-                    ((flags & ZS_FUSED_COST_SCALED) ? FUSED_COST_SCALED : 0),
-                false, as_stream(stream)};
-    ZS_REQUIRE(persistent_grid(B) <= ZS_FUSED_LOSS_MAX_GRID, ZS_ERR_UNSUPPORTED);
-    c.loss_out = loss_out;
-    c.ticket = (unsigned*)workspace;
-    c.poisson = true;
-    return fused_launch(c);
+    return fused_entry(true, true, estimator, loss_out, workspace, cost, drate, dlogp, dlogq, logpx_out, rate, x,
+                       logp_other, logq, K, B, X, grad_scale, flags, stream);
 }
 
 /* Debug hooks (not used by the Python package's hot path). */

@@ -16,6 +16,7 @@
 // Anything else returns ZS_ERR_UNSUPPORTED and the caller composes the general kernels of zs_nodes.cu.
 #include <initializer_list>
 #include <stdlib.h>
+#include <type_traits>
 
 #include "zs_common.cuh"
 #include "zs_philox.cuh"
@@ -794,48 +795,23 @@ static bool latent_fwd_rows_f32(float* z, float* logq, float* logp, const float*
 
 // float / KBCAST / 32-bit indexable shapes go to k_latent_fwd_fast; returns false when the shape does not qualify
 template <typename T, int FAM>
-static bool launch_latent_fwd_fast(dim3, T*, T*, T*, const T*, int, const T*, const T*, const T*, const T*, int64_t,
-                                   int64_t, int64_t, int, int64_t, uint64_t, uint64_t, unsigned long long*,
-                                   cudaStream_t, unsigned char*) {
+static bool launch_latent_fwd_fast(dim3 grid, T* z, T* logq, T* logp, const T* a, int a_mode, const T* b, const T* pa,
+                                   const T* pb, const T* noise_in, int64_t K, int64_t M, int64_t E4, int RW, int64_t KS,
+                                   uint64_t seed, uint64_t offset, unsigned long long* rs, cudaStream_t st,
+                                   unsigned char* zbits) {
+    if constexpr (std::is_same<T, float>::value) {
+        if (a_mode != ZS_KBCAST || K * M * E4 >= ((int64_t)1 << 31) || K * M >= ((int64_t)1 << 31)) return false;
+        if (latent_fwd_rows_f32<FAM>(z, logq, logp, a, a_mode, b, pa, pb, noise_in, K, M, E4, seed, offset, rs, st,
+                                     zbits))
+            return true;
+        const unsigned inv = (unsigned)((65536 + E4 - 1) / E4);
+        const bool stdp = FAM == FAM_NORMAL ? (pa == nullptr && pb == nullptr) : pa == nullptr;
+        launch_pdl(PDL_LATENT_FWD, stdp ? k_latent_fwd_fast<FAM, true> : k_latent_fwd_fast<FAM, false>, grid,
+                   dim3(LF_WARPS * 32), 0, st, z, logq, logp, a, b, pa, pb, noise_in, (int)K, (int)M, (int)E4, RW,
+                   (int)KS, inv, seed, offset, rs, zbits);
+        return true;
+    }
     return false;
-}
-template <>
-bool launch_latent_fwd_fast<float, FAM_NORMAL>(dim3 grid, float* z, float* logq, float* logp, const float* a, int a_mode,
-                                               const float* b, const float* pa, const float* pb, const float* noise_in,
-                                               int64_t K, int64_t M, int64_t E4, int RW, int64_t KS, uint64_t seed,
-                                               uint64_t offset, unsigned long long* rs, cudaStream_t st,
-                                               unsigned char* zbits) {
-    if (a_mode != ZS_KBCAST || K * M * E4 >= ((int64_t)1 << 31) || K * M >= ((int64_t)1 << 31)) return false;
-    if (latent_fwd_rows_f32<FAM_NORMAL>(z, logq, logp, a, a_mode, b, pa, pb, noise_in, K, M, E4, seed, offset, rs, st,
-                                        zbits))
-        return true;
-    const unsigned inv = (unsigned)((65536 + E4 - 1) / E4);
-    if (pa == nullptr && pb == nullptr)
-        launch_pdl(PDL_LATENT_FWD, k_latent_fwd_fast<FAM_NORMAL, true>, grid, dim3(LF_WARPS * 32), 0, st, z, logq, logp, a, b, pa, pb,
-                   noise_in, (int)K, (int)M, (int)E4, RW, (int)KS, inv, seed, offset, rs, zbits);
-    else
-        launch_pdl(PDL_LATENT_FWD, k_latent_fwd_fast<FAM_NORMAL, false>, grid, dim3(LF_WARPS * 32), 0, st, z, logq, logp, a, b, pa, pb,
-                   noise_in, (int)K, (int)M, (int)E4, RW, (int)KS, inv, seed, offset, rs, zbits);
-    return true;
-}
-template <>
-bool launch_latent_fwd_fast<float, FAM_BERNOULLI>(dim3 grid, float* z, float* logq, float* logp, const float* a,
-                                                  int a_mode, const float* b, const float* pa, const float* pb,
-                                                  const float* noise_in, int64_t K, int64_t M, int64_t E4, int RW,
-                                                  int64_t KS, uint64_t seed, uint64_t offset, unsigned long long* rs,
-                                                  cudaStream_t st, unsigned char* zbits) {
-    if (a_mode != ZS_KBCAST || K * M * E4 >= ((int64_t)1 << 31) || K * M >= ((int64_t)1 << 31)) return false;
-    if (latent_fwd_rows_f32<FAM_BERNOULLI>(z, logq, logp, a, a_mode, b, pa, pb, noise_in, K, M, E4, seed, offset, rs, st,
-                                           zbits))
-        return true;
-    const unsigned inv = (unsigned)((65536 + E4 - 1) / E4);
-    if (pa == nullptr)
-        launch_pdl(PDL_LATENT_FWD, k_latent_fwd_fast<FAM_BERNOULLI, true>, grid, dim3(LF_WARPS * 32), 0, st, z, logq, logp, a, b, pa, pb,
-                   noise_in, (int)K, (int)M, (int)E4, RW, (int)KS, inv, seed, offset, rs, zbits);
-    else
-        launch_pdl(PDL_LATENT_FWD, k_latent_fwd_fast<FAM_BERNOULLI, false>, grid, dim3(LF_WARPS * 32), 0, st, z, logq, logp, a, b, pa, pb,
-                   noise_in, (int)K, (int)M, (int)E4, RW, (int)KS, inv, seed, offset, rs, zbits);
-    return true;
 }
 
 template <typename T, int FAM>
@@ -1050,16 +1026,11 @@ __global__ void __launch_bounds__(LB_X_MAX* LB_Y_MAX, LBF_U > 4 ? 2 : 4)
     }
 }
 
-template <typename T, int FAM>
-static bool launch_latent_bwd_fast(void*, void*, const void*, const void*, const void*, const void*, const void*, int,
-                                   const void*, const void*, const void*, int, int64_t, int64_t, int64_t, cudaStream_t,
-                                   const void*) {
-    return false;
-}
+// float / KBCAST / 32-bit indexable shapes go to k_latent_bwd_fast; returns false when the shape does not qualify
 template <int FAM>
-static bool latent_bwd_fast_f32(void* da, void* db, const void* gq, const void* gp, const void* dz_up, const void* z,
-                                const void* a, int a_mode, const void* b, const void* pa, const void* pb, int reparam,
-                                int64_t K, int64_t M, int64_t E, cudaStream_t st, const void* zbits) {
+static bool launch_latent_bwd_fast(void* da, void* db, const void* gq, const void* gp, const void* dz_up, const void* z,
+                                   const void* a, int a_mode, const void* b, const void* pa, const void* pb, int reparam,
+                                   int64_t K, int64_t M, int64_t E, cudaStream_t st, const void* zbits) {
     if (a_mode != ZS_KBCAST || K * M * E >= ((int64_t)1 << 31) || da == nullptr || (FAM == FAM_NORMAL && db == nullptr))
         return false;
     const int64_t ME4 = (M * E) >> 2;
@@ -1100,28 +1071,14 @@ static bool latent_bwd_fast_f32(void* da, void* db, const void* gq, const void* 
                (const float*)pb, reparam, (int)K, (int)M, (int)E, (const unsigned char*)zbits);
     return true;
 }
-template <>
-bool launch_latent_bwd_fast<float, FAM_NORMAL>(void* da, void* db, const void* gq, const void* gp, const void* dz_up,
-                                               const void* z, const void* a, int a_mode, const void* b, const void* pa,
-                                               const void* pb, int reparam, int64_t K, int64_t M, int64_t E,
-                                               cudaStream_t st, const void* zbits) {
-    return latent_bwd_fast_f32<FAM_NORMAL>(da, db, gq, gp, dz_up, z, a, a_mode, b, pa, pb, reparam, K, M, E, st, zbits);
-}
-template <>
-bool launch_latent_bwd_fast<float, FAM_BERNOULLI>(void* da, void* db, const void* gq, const void* gp, const void* dz_up,
-                                                  const void* z, const void* a, int a_mode, const void* b,
-                                                  const void* pa, const void* pb, int reparam, int64_t K, int64_t M,
-                                                  int64_t E, cudaStream_t st, const void* zbits) {
-    return latent_bwd_fast_f32<FAM_BERNOULLI>(da, db, gq, gp, dz_up, z, a, a_mode, b, pa, pb, reparam, K, M, E, st, zbits);
-}
 
 template <typename T, int FAM>
 static int launch_latent_bwd(void* da, void* db, const void* gq, const void* gp, const void* dz_up, const void* z,
                              const void* a, int a_mode, const void* b, int b_mode, const void* pa, const void* pb,
                              int reparam, int64_t K, int64_t M, int64_t E, zs_stream_t stream,
                              const void* zbits = nullptr) {
-    if (launch_latent_bwd_fast<T, FAM>(da, db, gq, gp, dz_up, z, a, a_mode, b, pa, pb, reparam, K, M, E,
-                                       as_stream(stream), zbits)) {
+    if (std::is_same<T, float>::value && launch_latent_bwd_fast<FAM>(da, db, gq, gp, dz_up, z, a, a_mode, b, pa, pb,
+                                                                     reparam, K, M, E, as_stream(stream), zbits)) {
         ZS_LAUNCH_CHECK("k_latent_bwd_fast");
         return ZS_OK;
     }
@@ -1169,19 +1126,12 @@ int zs_normal_latent_fwd(int dtype, void* z, void* logq, void* logp, const void*
     int rc = latent_args_ok(mean, mean_mode, std, std_mode, FAM_NORMAL, E, {z, mean, std, prior_mean, prior_std, eps_in});
     if (rc != ZS_OK) return rc;
     if (K * M == 0) return ZS_OK;
-    if (dtype == ZS_F32)
-        return launch_latent_fwd<float, FAM_NORMAL>((float*)z, (float*)logq, (float*)logp, (const float*)mean,
-                                                    mean_mode, (const float*)std, std_mode, (const float*)prior_mean,
-                                                    (const float*)prior_std, (const float*)eps_in, K, M, E, seed,
-                                                    offset, (unsigned long long*)rng_state, as_stream(stream));
-    if (dtype == ZS_F64)
-        return launch_latent_fwd<double, FAM_NORMAL>((double*)z, (double*)logq, (double*)logp, (const double*)mean,
-                                                     mean_mode, (const double*)std, std_mode,
-                                                     (const double*)prior_mean, (const double*)prior_std,
-                                                     (const double*)eps_in, K, M, E, seed, offset,
-                                                     (unsigned long long*)rng_state, as_stream(stream));
-    set_last_error_msg("dtype must be ZS_F32 or ZS_F64");
-    return ZS_ERR_DTYPE;
+    ZS_DTYPE_SWITCH(dtype, {
+        return launch_latent_fwd<T, FAM_NORMAL>((T*)z, (T*)logq, (T*)logp, (const T*)mean, mean_mode, (const T*)std,
+                                                std_mode, (const T*)prior_mean, (const T*)prior_std, (const T*)eps_in,
+                                                K, M, E, seed, offset, (unsigned long long*)rng_state,
+                                                as_stream(stream));
+    })
 }
 
 int zs_bernoulli_latent_fwd(int dtype, void* z, void* logq, void* logp, const void* probs, int probs_mode,
@@ -1192,20 +1142,12 @@ int zs_bernoulli_latent_fwd(int dtype, void* z, void* logq, void* logp, const vo
     int rc = latent_args_ok(probs, probs_mode, nullptr, probs_mode, FAM_BERNOULLI, E, {z, probs, prior_probs, u_in});
     if (rc != ZS_OK) return rc;
     if (K * M == 0) return ZS_OK;
-    if (dtype == ZS_F32)
-        return launch_latent_fwd<float, FAM_BERNOULLI>((float*)z, (float*)logq, (float*)logp, (const float*)probs,
-                                                       probs_mode, nullptr, probs_mode, (const float*)prior_probs,
-                                                       nullptr, (const float*)u_in, K, M, E, seed, offset,
-                                                       (unsigned long long*)rng_state, as_stream(stream),
-                                                       (unsigned char*)zbits);
-    if (dtype == ZS_F64)
-        return launch_latent_fwd<double, FAM_BERNOULLI>((double*)z, (double*)logq, (double*)logp,
-                                                        (const double*)probs, probs_mode, nullptr, probs_mode,
-                                                        (const double*)prior_probs, nullptr, (const double*)u_in, K,
-                                                        M, E, seed, offset, (unsigned long long*)rng_state,
-                                                        as_stream(stream));
-    set_last_error_msg("dtype must be ZS_F32 or ZS_F64");
-    return ZS_ERR_DTYPE;
+    ZS_DTYPE_SWITCH(dtype, {
+        return launch_latent_fwd<T, FAM_BERNOULLI>((T*)z, (T*)logq, (T*)logp, (const T*)probs, probs_mode, nullptr,
+                                                   probs_mode, (const T*)prior_probs, nullptr, (const T*)u_in, K, M, E,
+                                                   seed, offset, (unsigned long long*)rng_state, as_stream(stream),
+                                                   (unsigned char*)zbits);
+    })
 }
 
 int zs_normal_latent_bwd(int dtype, void* dmean, void* dstd, const void* dlogq, const void* dlogp, const void* dz_up,
@@ -1217,15 +1159,10 @@ int zs_normal_latent_bwd(int dtype, void* dmean, void* dstd, const void* dlogq, 
                             {dmean, dstd, dz_up, z, mean, std, prior_mean, prior_std});
     if (rc != ZS_OK) return rc;
     if (K * M == 0 || (!dmean && !dstd)) return ZS_OK;
-    if (dtype == ZS_F32)
-        return launch_latent_bwd<float, FAM_NORMAL>(dmean, dstd, dlogq, dlogp, dz_up, z, mean, mean_mode, std,
-                                                    std_mode, prior_mean, prior_std, reparameterized, K, M, E, stream);
-    if (dtype == ZS_F64)
-        return launch_latent_bwd<double, FAM_NORMAL>(dmean, dstd, dlogq, dlogp, dz_up, z, mean, mean_mode, std,
-                                                     std_mode, prior_mean, prior_std, reparameterized, K, M, E,
-                                                     stream);
-    set_last_error_msg("dtype must be ZS_F32 or ZS_F64");
-    return ZS_ERR_DTYPE;
+    ZS_DTYPE_SWITCH(dtype, {
+        return launch_latent_bwd<T, FAM_NORMAL>(dmean, dstd, dlogq, dlogp, dz_up, z, mean, mean_mode, std, std_mode,
+                                                prior_mean, prior_std, reparameterized, K, M, E, stream);
+    })
 }
 
 int zs_bernoulli_latent_bwd(int dtype, void* dprobs, const void* dlogq, const void* z, const void* probs,
@@ -1234,15 +1171,10 @@ int zs_bernoulli_latent_bwd(int dtype, void* dprobs, const void* dlogq, const vo
     int rc = latent_args_ok(probs, probs_mode, nullptr, probs_mode, FAM_BERNOULLI, E, {dprobs, z, probs});
     if (rc != ZS_OK) return rc;
     if (K * M == 0) return ZS_OK;
-    if (dtype == ZS_F32)
-        return launch_latent_bwd<float, FAM_BERNOULLI>(dprobs, nullptr, dlogq, nullptr, nullptr, z, probs, probs_mode,
-                                                       nullptr, probs_mode, nullptr, nullptr, 0, K, M, E, stream, zbits);
-    if (dtype == ZS_F64)
-        return launch_latent_bwd<double, FAM_BERNOULLI>(dprobs, nullptr, dlogq, nullptr, nullptr, z, probs,
-                                                        probs_mode, nullptr, probs_mode, nullptr, nullptr, 0, K, M, E,
-                                                        stream);
-    set_last_error_msg("dtype must be ZS_F32 or ZS_F64");
-    return ZS_ERR_DTYPE;
+    ZS_DTYPE_SWITCH(dtype, {
+        return launch_latent_bwd<T, FAM_BERNOULLI>(dprobs, nullptr, dlogq, nullptr, nullptr, z, probs, probs_mode,
+                                                   nullptr, probs_mode, nullptr, nullptr, 0, K, M, E, stream, zbits);
+    })
 }
 
 }  // extern "C"

@@ -1165,6 +1165,74 @@ static int dispatch_bwd(T* dx, T* da, T* db, const T* g, Operand<T> x, Operand<T
     return launch_rows_bwd<T, Op, 32>(dx, da, db, g, x, a, b, K, M, E, st);
 }
 
+// ---------------------------------------------------------------------------
+// C-ABI entry helpers of the row log-density entry points: argument checks, dtype switch, operands.  Bernoulli, its
+// logits form and Poisson have one parameter; their callers pass b = nullptr, bm = ZS_SCALAR.
+// ---------------------------------------------------------------------------
+template <template <typename> class Op>
+constexpr bool kOneParam = false;
+template <>
+constexpr bool kOneParam<BernoulliOp> = true;
+template <>
+constexpr bool kOneParam<BernoulliLogitsOp> = true;
+template <>
+constexpr bool kOneParam<PoissonOp> = true;
+
+template <template <typename> class Op>
+static int rows_logprob_fwd(int dtype, void* out, const void* x, int xm, const void* a, int am, const void* b, int bm,
+                            int64_t K, int64_t M, int64_t E, zs_stream_t stream) {
+    ZS_REQUIRE(out && x && a && (b || kOneParam<Op>) && K >= 0 && M >= 0 && E >= 1, ZS_ERR_ARG);
+    ZS_REQUIRE(valid_mode(xm) && valid_mode(am) && valid_mode(bm), ZS_ERR_ARG);
+    ZS_DTYPE_SWITCH(dtype, {
+        return dispatch_rows_fwd<T, Op<T>>((T*)out, Operand<T>{(const T*)x, xm}, Operand<T>{(const T*)a, am},
+                                           Operand<T>{(const T*)b, bm}, K, M, E, as_stream(stream));
+    })
+}
+
+template <template <typename> class Op>
+static int rows_logprob_bwd(int dtype, void* dx, void* da, void* db, const void* g, const void* x, int xm,
+                            const void* a, int am, const void* b, int bm, int64_t K, int64_t M, int64_t E,
+                            zs_stream_t stream) {
+    ZS_REQUIRE(g && x && a && (b || kOneParam<Op>) && K >= 0 && M >= 0 && E >= 1, ZS_ERR_ARG);
+    ZS_REQUIRE(valid_mode(xm) && valid_mode(am) && valid_mode(bm), ZS_ERR_ARG);
+    if (!dx && !da && !db) return ZS_OK;
+    ZS_DTYPE_SWITCH(dtype, {
+        return dispatch_bwd<T, Op<T>>((T*)dx, (T*)da, (T*)db, (const T*)g, Operand<T>{(const T*)x, xm},
+                                      Operand<T>{(const T*)a, am}, Operand<T>{(const T*)b, bm}, K, M, E,
+                                      as_stream(stream));
+    })
+}
+
+// f(OpTag<Op>{}) with the per-element Op of a zs_locscale_logprob_* family; ZS_ERR_ARG for an unknown family
+template <template <typename> class FamilyOp>
+struct OpTag {
+    template <typename T>
+    using Op = FamilyOp<T>;
+};
+template <typename F>
+static int with_locscale_op(int family, F&& f) {
+    switch (family) {
+        case ZS_FAM_LOGISTIC: return f(OpTag<LogisticOp>{});
+        case ZS_FAM_LAPLACE: return f(OpTag<LaplaceOp>{});
+        case ZS_FAM_UNIFORM: return f(OpTag<UniformOp>{});  // loc = low, scale = high
+        case ZS_FAM_BETA: return f(OpTag<BetaOp>{});        // loc = alpha, scale = beta
+    }
+    set_last_error_msg("family must be ZS_FAM_LOGISTIC, ZS_FAM_LAPLACE, ZS_FAM_UNIFORM or ZS_FAM_BETA");
+    return ZS_ERR_ARG;
+}
+
+// f(integral_constant<int, NOISE_*>{}) with the sampler noise of a zs_locscale_sample* family; ZS_ERR_ARG for any other
+template <typename F>
+static int with_locscale_noise(int family, F&& f) {
+    switch (family) {
+        case ZS_FAM_LOGISTIC: return f(std::integral_constant<int, NOISE_LOGISTIC>{});
+        case ZS_FAM_LAPLACE: return f(std::integral_constant<int, NOISE_LAPLACE>{});
+        case ZS_FAM_UNIFORM: return f(std::integral_constant<int, NOISE_UNIFORM>{});
+    }
+    set_last_error_msg("family must be ZS_FAM_LOGISTIC, ZS_FAM_LAPLACE or ZS_FAM_UNIFORM");
+    return ZS_ERR_ARG;
+}
+
 }  // namespace zs
 
 using namespace zs;
@@ -1176,18 +1244,6 @@ __global__ void k_rng_state_init(unsigned long long* st, unsigned long long offs
 static inline unsigned long long* rs_ptr(const void* p) {
     return reinterpret_cast<unsigned long long*>(const_cast<void*>(p));
 }
-
-#define ZS_DTYPE_SWITCH(dtype, ...)              \
-    if ((dtype) == ZS_F32) {                     \
-        using T = float;                         \
-        __VA_ARGS__                              \
-    } else if ((dtype) == ZS_F64) {              \
-        using T = double;                        \
-        __VA_ARGS__                              \
-    } else {                                     \
-        set_last_error_msg("dtype must be ZS_F32 or ZS_F64"); \
-        return ZS_ERR_DTYPE;                     \
-    }
 
 extern "C" {
 
@@ -1276,26 +1332,14 @@ int zs_normal_sample_bwd(int dtype, void* dmean, int mean_mode, void* dstd, int 
 
 int zs_normal_logprob_fwd(int dtype, void* out, const void* x, int x_mode, const void* mean, int mean_mode,
                           const void* std, int std_mode, int64_t K, int64_t M, int64_t E, zs_stream_t stream) {
-    ZS_REQUIRE(out && x && mean && std && K >= 0 && M >= 0 && E >= 1, ZS_ERR_ARG);
-    ZS_REQUIRE(valid_mode(x_mode) && valid_mode(mean_mode) && valid_mode(std_mode), ZS_ERR_ARG);
-    ZS_DTYPE_SWITCH(dtype, {
-        return dispatch_rows_fwd<T, NormalOp<T>>((T*)out, Operand<T>{(const T*)x, x_mode},
-                                                 Operand<T>{(const T*)mean, mean_mode},
-                                                 Operand<T>{(const T*)std, std_mode}, K, M, E, as_stream(stream));
-    })
+    return rows_logprob_fwd<NormalOp>(dtype, out, x, x_mode, mean, mean_mode, std, std_mode, K, M, E, stream);
 }
 
 int zs_normal_logprob_bwd(int dtype, void* dx, void* dmean, void* dstd, const void* g, const void* x, int x_mode,
                           const void* mean, int mean_mode, const void* std, int std_mode, int64_t K, int64_t M,
                           int64_t E, zs_stream_t stream) {
-    ZS_REQUIRE(g && x && mean && std && K >= 0 && M >= 0 && E >= 1, ZS_ERR_ARG);
-    ZS_REQUIRE(valid_mode(x_mode) && valid_mode(mean_mode) && valid_mode(std_mode), ZS_ERR_ARG);
-    if (!dx && !dmean && !dstd) return ZS_OK;
-    ZS_DTYPE_SWITCH(dtype, {
-        return dispatch_bwd<T, NormalOp<T>>((T*)dx, (T*)dmean, (T*)dstd, (const T*)g, Operand<T>{(const T*)x, x_mode},
-                                            Operand<T>{(const T*)mean, mean_mode},
-                                            Operand<T>{(const T*)std, std_mode}, K, M, E, as_stream(stream));
-    })
+    return rows_logprob_bwd<NormalOp>(dtype, dx, dmean, dstd, g, x, x_mode, mean, mean_mode, std, std_mode, K, M, E,
+                                      stream);
 }
 
 int zs_bernoulli_sample(int dtype, void* out, const void* probs, int probs_mode, const void* u_in, int64_t K,
@@ -1320,26 +1364,13 @@ int zs_bernoulli_sample(int dtype, void* out, const void* probs, int probs_mode,
 
 int zs_bernoulli_logpmf_fwd(int dtype, void* out, const void* x, int x_mode, const void* probs, int probs_mode,
                             int64_t K, int64_t M, int64_t E, zs_stream_t stream) {
-    ZS_REQUIRE(out && x && probs && K >= 0 && M >= 0 && E >= 1, ZS_ERR_ARG);
-    ZS_REQUIRE(valid_mode(x_mode) && valid_mode(probs_mode), ZS_ERR_ARG);
-    ZS_DTYPE_SWITCH(dtype, {
-        return dispatch_rows_fwd<T, BernoulliOp<T>>((T*)out, Operand<T>{(const T*)x, x_mode},
-                                                    Operand<T>{(const T*)probs, probs_mode},
-                                                    Operand<T>{nullptr, ZS_SCALAR}, K, M, E, as_stream(stream));
-    })
+    return rows_logprob_fwd<BernoulliOp>(dtype, out, x, x_mode, probs, probs_mode, nullptr, ZS_SCALAR, K, M, E, stream);
 }
 
 int zs_bernoulli_logpmf_bwd(int dtype, void* dx, void* dprobs, const void* g, const void* x, int x_mode,
                             const void* probs, int probs_mode, int64_t K, int64_t M, int64_t E, zs_stream_t stream) {
-    ZS_REQUIRE(g && x && probs && K >= 0 && M >= 0 && E >= 1, ZS_ERR_ARG);
-    ZS_REQUIRE(valid_mode(x_mode) && valid_mode(probs_mode), ZS_ERR_ARG);
-    if (!dx && !dprobs) return ZS_OK;
-    ZS_DTYPE_SWITCH(dtype, {
-        return dispatch_bwd<T, BernoulliOp<T>>((T*)dx, (T*)dprobs, (T*)nullptr, (const T*)g,
-                                               Operand<T>{(const T*)x, x_mode},
-                                               Operand<T>{(const T*)probs, probs_mode},
-                                               Operand<T>{nullptr, ZS_SCALAR}, K, M, E, as_stream(stream));
-    })
+    return rows_logprob_bwd<BernoulliOp>(dtype, dx, dprobs, nullptr, g, x, x_mode, probs, probs_mode, nullptr,
+                                         ZS_SCALAR, K, M, E, stream);
 }
 
 /* ---- location-scale families beyond Normal (SURVEY 8(f)-4) ------------------------------------------------ */
@@ -1349,25 +1380,17 @@ int zs_locscale_sample(int dtype, int family, void* z, const void* loc, int loc_
     ZS_REQUIRE(z && loc && scale && K >= 0 && N >= 0, ZS_ERR_ARG);
     if (u_in) rng_state = rng_snapshot = nullptr;
     ZS_REQUIRE(valid_mode(loc_mode) && valid_mode(scale_mode), ZS_ERR_ARG);
-    ZS_REQUIRE(family == ZS_FAM_LOGISTIC || family == ZS_FAM_LAPLACE || family == ZS_FAM_UNIFORM, ZS_ERR_ARG);
-    if (K * N == 0) return ZS_OK;
-    const int grid = grid_for((K * N + 3) / 4, 256);
-    ZS_DTYPE_SWITCH(dtype, {
-        if (family == ZS_FAM_LOGISTIC)
-            k_normal_sample<T, false, NOISE_LOGISTIC><<<grid, 256, 0, as_stream(stream)>>>(
-                (T*)z, (const T*)loc, loc_mode, (const T*)scale, scale_mode, (const T*)u_in, (T*)nullptr, K, N, seed, offset,
-                rs_ptr(rng_state), rs_ptr(rng_snapshot));
-        else if (family == ZS_FAM_UNIFORM)
-            k_normal_sample<T, false, NOISE_UNIFORM><<<grid, 256, 0, as_stream(stream)>>>(
-                (T*)z, (const T*)loc, loc_mode, (const T*)scale, scale_mode, (const T*)u_in, (T*)nullptr, K, N, seed, offset,
-                rs_ptr(rng_state), rs_ptr(rng_snapshot));
-        else
-            k_normal_sample<T, false, NOISE_LAPLACE><<<grid, 256, 0, as_stream(stream)>>>(
-                (T*)z, (const T*)loc, loc_mode, (const T*)scale, scale_mode, (const T*)u_in, (T*)nullptr, K, N, seed, offset,
-                rs_ptr(rng_state), rs_ptr(rng_snapshot));
-    })
-    ZS_LAUNCH_CHECK("k_normal_sample<locscale>");
-    return ZS_OK;
+    return with_locscale_noise(family, [&](auto noise) -> int {
+        if (K * N == 0) return ZS_OK;
+        const int grid = grid_for((K * N + 3) / 4, 256);
+        ZS_DTYPE_SWITCH(dtype, {
+            k_normal_sample<T, false, decltype(noise)::value><<<grid, 256, 0, as_stream(stream)>>>(
+                (T*)z, (const T*)loc, loc_mode, (const T*)scale, scale_mode, (const T*)u_in, (T*)nullptr, K, N, seed,
+                offset, rs_ptr(rng_state), rs_ptr(rng_snapshot));
+        })
+        ZS_LAUNCH_CHECK("k_normal_sample<locscale>");
+        return ZS_OK;
+    });
 }
 
 int zs_locscale_sample_bwd(int dtype, int family, void* dloc, int loc_mode, void* dscale, int scale_mode, const void* dz,
@@ -1375,110 +1398,53 @@ int zs_locscale_sample_bwd(int dtype, int family, void* dloc, int loc_mode, void
                            zs_stream_t stream) {
     ZS_REQUIRE(dz && K >= 0 && N >= 0, ZS_ERR_ARG);
     ZS_REQUIRE(valid_mode(loc_mode) && valid_mode(scale_mode), ZS_ERR_ARG);
-    ZS_REQUIRE(family == ZS_FAM_LOGISTIC || family == ZS_FAM_LAPLACE || family == ZS_FAM_UNIFORM, ZS_ERR_ARG);
-    if ((dloc && loc_mode == ZS_SCALAR) || (dscale && scale_mode == ZS_SCALAR)) {
-        set_last_error_msg("SCALAR-mode gradients are not produced by the kernels; expand the operand");
-        return ZS_ERR_UNSUPPORTED;
-    }
-    if (K * N == 0 || (!dloc && !dscale)) return ZS_OK;
-    dim3 block(KR_X, KR_Y);
-    const int64_t grid = (N + KR_X - 1) / KR_X;
-    ZS_REQUIRE(grid < (int64_t)2147483647, ZS_ERR_UNSUPPORTED);
-    ZS_DTYPE_SWITCH(dtype, {
-        if (family == ZS_FAM_LOGISTIC)
-            k_normal_sample_bwd<T, NOISE_LOGISTIC><<<(unsigned)grid, block, 0, as_stream(stream)>>>(
+    return with_locscale_noise(family, [&](auto noise) -> int {
+        if ((dloc && loc_mode == ZS_SCALAR) || (dscale && scale_mode == ZS_SCALAR)) {
+            set_last_error_msg("SCALAR-mode gradients are not produced by the kernels; expand the operand");
+            return ZS_ERR_UNSUPPORTED;
+        }
+        if (K * N == 0 || (!dloc && !dscale)) return ZS_OK;
+        dim3 block(KR_X, KR_Y);
+        const int64_t grid = (N + KR_X - 1) / KR_X;
+        ZS_REQUIRE(grid < (int64_t)2147483647, ZS_ERR_UNSUPPORTED);
+        ZS_DTYPE_SWITCH(dtype, {
+            k_normal_sample_bwd<T, decltype(noise)::value><<<(unsigned)grid, block, 0, as_stream(stream)>>>(
                 (T*)dloc, loc_mode, (T*)dscale, scale_mode, (const T*)dz, (const T*)u, K, N, seed, offset,
                 u ? nullptr : rs_ptr(rng_state));
-        else if (family == ZS_FAM_UNIFORM)
-            k_normal_sample_bwd<T, NOISE_UNIFORM><<<(unsigned)grid, block, 0, as_stream(stream)>>>(
-                (T*)dloc, loc_mode, (T*)dscale, scale_mode, (const T*)dz, (const T*)u, K, N, seed, offset,
-                u ? nullptr : rs_ptr(rng_state));
-        else
-            k_normal_sample_bwd<T, NOISE_LAPLACE><<<(unsigned)grid, block, 0, as_stream(stream)>>>(
-                (T*)dloc, loc_mode, (T*)dscale, scale_mode, (const T*)dz, (const T*)u, K, N, seed, offset,
-                u ? nullptr : rs_ptr(rng_state));
-    })
-    ZS_LAUNCH_CHECK("k_normal_sample_bwd<locscale>");
-    return ZS_OK;
+        })
+        ZS_LAUNCH_CHECK("k_normal_sample_bwd<locscale>");
+        return ZS_OK;
+    });
 }
 
 int zs_locscale_logprob_fwd(int dtype, int family, void* out, const void* x, int x_mode, const void* loc, int loc_mode,
                             const void* scale, int scale_mode, int64_t K, int64_t M, int64_t E, zs_stream_t stream) {
-    ZS_REQUIRE(out && x && loc && scale && K >= 0 && M >= 0 && E >= 1, ZS_ERR_ARG);
-    ZS_REQUIRE(valid_mode(x_mode) && valid_mode(loc_mode) && valid_mode(scale_mode), ZS_ERR_ARG);
-    ZS_REQUIRE(family == ZS_FAM_LOGISTIC || family == ZS_FAM_LAPLACE || family == ZS_FAM_UNIFORM ||
-                   family == ZS_FAM_BETA,
-               ZS_ERR_ARG);
-    ZS_DTYPE_SWITCH(dtype, {
-        if (family == ZS_FAM_BETA)  // loc = alpha, scale = beta
-            return dispatch_rows_fwd<T, BetaOp<T>>((T*)out, Operand<T>{(const T*)x, x_mode},
-                                                   Operand<T>{(const T*)loc, loc_mode},
-                                                   Operand<T>{(const T*)scale, scale_mode}, K, M, E, as_stream(stream));
-        if (family == ZS_FAM_LOGISTIC)
-            return dispatch_rows_fwd<T, LogisticOp<T>>((T*)out, Operand<T>{(const T*)x, x_mode},
-                                                       Operand<T>{(const T*)loc, loc_mode},
-                                                       Operand<T>{(const T*)scale, scale_mode}, K, M, E, as_stream(stream));
-        if (family == ZS_FAM_UNIFORM)  // loc = low, scale = high
-            return dispatch_rows_fwd<T, UniformOp<T>>((T*)out, Operand<T>{(const T*)x, x_mode},
-                                                      Operand<T>{(const T*)loc, loc_mode},
-                                                      Operand<T>{(const T*)scale, scale_mode}, K, M, E, as_stream(stream));
-        return dispatch_rows_fwd<T, LaplaceOp<T>>((T*)out, Operand<T>{(const T*)x, x_mode},
-                                                  Operand<T>{(const T*)loc, loc_mode},
-                                                  Operand<T>{(const T*)scale, scale_mode}, K, M, E, as_stream(stream));
-    })
+    return with_locscale_op(family, [&](auto tag) {
+        return rows_logprob_fwd<decltype(tag)::template Op>(dtype, out, x, x_mode, loc, loc_mode, scale, scale_mode, K,
+                                                            M, E, stream);
+    });
 }
 
 int zs_locscale_logprob_bwd(int dtype, int family, void* dx, void* dloc, void* dscale, const void* g, const void* x,
                             int x_mode, const void* loc, int loc_mode, const void* scale, int scale_mode, int64_t K,
                             int64_t M, int64_t E, zs_stream_t stream) {
-    ZS_REQUIRE(g && x && loc && scale && K >= 0 && M >= 0 && E >= 1, ZS_ERR_ARG);
-    ZS_REQUIRE(valid_mode(x_mode) && valid_mode(loc_mode) && valid_mode(scale_mode), ZS_ERR_ARG);
-    ZS_REQUIRE(family == ZS_FAM_LOGISTIC || family == ZS_FAM_LAPLACE || family == ZS_FAM_UNIFORM ||
-                   family == ZS_FAM_BETA,
-               ZS_ERR_ARG);
-    if (!dx && !dloc && !dscale) return ZS_OK;
-    ZS_DTYPE_SWITCH(dtype, {
-        if (family == ZS_FAM_BETA)
-            return dispatch_bwd<T, BetaOp<T>>((T*)dx, (T*)dloc, (T*)dscale, (const T*)g, Operand<T>{(const T*)x, x_mode},
-                                              Operand<T>{(const T*)loc, loc_mode},
-                                              Operand<T>{(const T*)scale, scale_mode}, K, M, E, as_stream(stream));
-        if (family == ZS_FAM_LOGISTIC)
-            return dispatch_bwd<T, LogisticOp<T>>((T*)dx, (T*)dloc, (T*)dscale, (const T*)g, Operand<T>{(const T*)x, x_mode},
-                                                  Operand<T>{(const T*)loc, loc_mode},
-                                                  Operand<T>{(const T*)scale, scale_mode}, K, M, E, as_stream(stream));
-        if (family == ZS_FAM_UNIFORM)
-            return dispatch_bwd<T, UniformOp<T>>((T*)dx, (T*)dloc, (T*)dscale, (const T*)g, Operand<T>{(const T*)x, x_mode},
-                                                 Operand<T>{(const T*)loc, loc_mode},
-                                                 Operand<T>{(const T*)scale, scale_mode}, K, M, E, as_stream(stream));
-        return dispatch_bwd<T, LaplaceOp<T>>((T*)dx, (T*)dloc, (T*)dscale, (const T*)g, Operand<T>{(const T*)x, x_mode},
-                                             Operand<T>{(const T*)loc, loc_mode},
-                                             Operand<T>{(const T*)scale, scale_mode}, K, M, E, as_stream(stream));
-    })
+    return with_locscale_op(family, [&](auto tag) {
+        return rows_logprob_bwd<decltype(tag)::template Op>(dtype, dx, dloc, dscale, g, x, x_mode, loc, loc_mode, scale,
+                                                            scale_mode, K, M, E, stream);
+    });
 }
 
 int zs_bernoulli_logits_logpmf_fwd(int dtype, void* out, const void* x, int x_mode, const void* logits, int logits_mode,
                                    int64_t K, int64_t M, int64_t E, zs_stream_t stream) {
-    ZS_REQUIRE(out && x && logits && K >= 0 && M >= 0 && E >= 1, ZS_ERR_ARG);
-    ZS_REQUIRE(valid_mode(x_mode) && valid_mode(logits_mode), ZS_ERR_ARG);
-    ZS_DTYPE_SWITCH(dtype, {
-        return dispatch_rows_fwd<T, BernoulliLogitsOp<T>>((T*)out, Operand<T>{(const T*)x, x_mode},
-                                                          Operand<T>{(const T*)logits, logits_mode},
-                                                          Operand<T>{nullptr, ZS_SCALAR}, K, M, E, as_stream(stream));
-    })
+    return rows_logprob_fwd<BernoulliLogitsOp>(dtype, out, x, x_mode, logits, logits_mode, nullptr, ZS_SCALAR, K, M, E,
+                                               stream);
 }
 
 int zs_bernoulli_logits_logpmf_bwd(int dtype, void* dx, void* dlogits, const void* g, const void* x, int x_mode,
                                    const void* logits, int logits_mode, int64_t K, int64_t M, int64_t E,
                                    zs_stream_t stream) {
-    ZS_REQUIRE(g && x && logits && K >= 0 && M >= 0 && E >= 1, ZS_ERR_ARG);
-    ZS_REQUIRE(valid_mode(x_mode) && valid_mode(logits_mode), ZS_ERR_ARG);
-    if (!dx && !dlogits) return ZS_OK;
-    ZS_DTYPE_SWITCH(dtype, {
-        return dispatch_bwd<T, BernoulliLogitsOp<T>>((T*)dx, (T*)dlogits, (T*)nullptr, (const T*)g,
-                                                     Operand<T>{(const T*)x, x_mode},
-                                                     Operand<T>{(const T*)logits, logits_mode},
-                                                     Operand<T>{nullptr, ZS_SCALAR}, K, M, E, as_stream(stream));
-    })
+    return rows_logprob_bwd<BernoulliLogitsOp>(dtype, dx, dlogits, nullptr, g, x, x_mode, logits, logits_mode, nullptr,
+                                               ZS_SCALAR, K, M, E, stream);
 }
 
 /* ---- Poisson stochastic node ---------------------------------------------------------------------------- */
@@ -1498,25 +1464,13 @@ int zs_poisson_sample(int dtype, void* out, const void* rate, int rate_mode, int
 
 int zs_poisson_logpmf_fwd(int dtype, void* out, const void* x, int x_mode, const void* rate, int rate_mode, int64_t K,
                           int64_t M, int64_t E, zs_stream_t stream) {
-    ZS_REQUIRE(out && x && rate && K >= 0 && M >= 0 && E >= 1, ZS_ERR_ARG);
-    ZS_REQUIRE(valid_mode(x_mode) && valid_mode(rate_mode), ZS_ERR_ARG);
-    ZS_DTYPE_SWITCH(dtype, {
-        return dispatch_rows_fwd<T, PoissonOp<T>>((T*)out, Operand<T>{(const T*)x, x_mode},
-                                                  Operand<T>{(const T*)rate, rate_mode},
-                                                  Operand<T>{nullptr, ZS_SCALAR}, K, M, E, as_stream(stream));
-    })
+    return rows_logprob_fwd<PoissonOp>(dtype, out, x, x_mode, rate, rate_mode, nullptr, ZS_SCALAR, K, M, E, stream);
 }
 
 int zs_poisson_logpmf_bwd(int dtype, void* drate, const void* g, const void* x, int x_mode, const void* rate,
                           int rate_mode, int64_t K, int64_t M, int64_t E, zs_stream_t stream) {
-    ZS_REQUIRE(g && x && rate && K >= 0 && M >= 0 && E >= 1, ZS_ERR_ARG);
-    ZS_REQUIRE(valid_mode(x_mode) && valid_mode(rate_mode), ZS_ERR_ARG);
-    if (!drate) return ZS_OK;
-    ZS_DTYPE_SWITCH(dtype, {
-        return dispatch_bwd<T, PoissonOp<T>>((T*)nullptr, (T*)drate, (T*)nullptr, (const T*)g,
-                                             Operand<T>{(const T*)x, x_mode}, Operand<T>{(const T*)rate, rate_mode},
-                                             Operand<T>{nullptr, ZS_SCALAR}, K, M, E, as_stream(stream));
-    })
+    return rows_logprob_bwd<PoissonOp>(dtype, nullptr, drate, nullptr, g, x, x_mode, rate, rate_mode, nullptr, ZS_SCALAR,
+                                       K, M, E, stream);
 }
 
 /* ---- Beta stochastic node (log-density: zs_locscale_logprob_* with ZS_FAM_BETA) ------------------------------ */

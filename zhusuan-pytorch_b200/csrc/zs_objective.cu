@@ -360,38 +360,14 @@ int zs_iw_objective(int dtype, int estimator, void* cost, void* dlogp, void* dlo
     const int64_t grid = (B + cols - 1) / cols;
     ZS_REQUIRE(grid < (int64_t)2147483647, ZS_ERR_UNSUPPORTED);
     cudaStream_t st = as_stream(stream);
-    if (dtype == ZS_F32) {
-        const size_t smem = OBJ_THREADS * (sizeof(double) + sizeof(long long));
-        if (estimator == ZS_EST_SGVB)
-            k_iw_objective<float, ZS_EST_SGVB><<<(unsigned)grid, block, smem, st>>>(
-                (float*)cost, (float*)dlogp, (float*)dlogq, (const float*)logp, (const float*)logq, (const float*)logp_extra, K, B,
-                (float)grad_scale, cols, slices);
-        else if (estimator == ZS_EST_ELBO)
-            k_iw_objective<float, ZS_EST_ELBO><<<(unsigned)grid, block, smem, st>>>(
-                (float*)cost, (float*)dlogp, (float*)dlogq, (const float*)logp, (const float*)logq, (const float*)logp_extra, K, B,
-                (float)grad_scale, cols, slices);
-        else
-            k_iw_objective<float, ZS_EST_VIMCO><<<(unsigned)grid, block, smem, st>>>(
-                (float*)cost, (float*)dlogp, (float*)dlogq, (const float*)logp, (const float*)logq, (const float*)logp_extra, K, B,
-                (float)grad_scale, cols, slices);
-    } else if (dtype == ZS_F64) {
-        const size_t smem = OBJ_THREADS * (sizeof(double) + sizeof(long long));
-        if (estimator == ZS_EST_SGVB)
-            k_iw_objective<double, ZS_EST_SGVB><<<(unsigned)grid, block, smem, st>>>(
-                (double*)cost, (double*)dlogp, (double*)dlogq, (const double*)logp, (const double*)logq, (const double*)logp_extra, K, B,
-                grad_scale, cols, slices);
-        else if (estimator == ZS_EST_ELBO)
-            k_iw_objective<double, ZS_EST_ELBO><<<(unsigned)grid, block, smem, st>>>(
-                (double*)cost, (double*)dlogp, (double*)dlogq, (const double*)logp, (const double*)logq, (const double*)logp_extra, K, B,
-                grad_scale, cols, slices);
-        else
-            k_iw_objective<double, ZS_EST_VIMCO><<<(unsigned)grid, block, smem, st>>>(
-                (double*)cost, (double*)dlogp, (double*)dlogq, (const double*)logp, (const double*)logq, (const double*)logp_extra, K, B,
-                grad_scale, cols, slices);
-    } else {
-        set_last_error_msg("dtype must be ZS_F32 or ZS_F64");
-        return ZS_ERR_DTYPE;
-    }
+    const size_t smem = OBJ_THREADS * (sizeof(double) + sizeof(long long));
+    ZS_DTYPE_SWITCH(dtype, {
+        auto kern = estimator == ZS_EST_SGVB   ? k_iw_objective<T, ZS_EST_SGVB>
+                    : estimator == ZS_EST_ELBO ? k_iw_objective<T, ZS_EST_ELBO>
+                                               : k_iw_objective<T, ZS_EST_VIMCO>;
+        kern<<<(unsigned)grid, block, smem, st>>>((T*)cost, (T*)dlogp, (T*)dlogq, (const T*)logp, (const T*)logq,
+                                                  (const T*)logp_extra, K, B, (T)grad_scale, cols, slices);
+    })
     ZS_LAUNCH_CHECK("k_iw_objective");
     return ZS_OK;
 }
@@ -406,26 +382,15 @@ static int lme_launch(int dtype, bool bwd, void* out, const void* g, const void*
     const int64_t grid = (B + cols - 1) / cols;
     ZS_REQUIRE(grid < (int64_t)2147483647, ZS_ERR_UNSUPPORTED);
     cudaStream_t st = as_stream(stream);
-    if (dtype == ZS_F32) {
-        const size_t smem = OBJ_THREADS * sizeof(float);
+    ZS_DTYPE_SWITCH(dtype, {
+        const size_t smem = OBJ_THREADS * sizeof(T);
         if (bwd)
-            k_log_mean_exp<float, true><<<(unsigned)grid, block, smem, st>>>((float*)out, (const float*)g,
-                                                                              (const float*)x, K, B, cols, slices);
+            k_log_mean_exp<T, true><<<(unsigned)grid, block, smem, st>>>((T*)out, (const T*)g, (const T*)x, K, B, cols,
+                                                                          slices);
         else
-            k_log_mean_exp<float, false><<<(unsigned)grid, block, smem, st>>>((float*)out, nullptr, (const float*)x,
-                                                                               K, B, cols, slices);
-    } else if (dtype == ZS_F64) {
-        const size_t smem = OBJ_THREADS * sizeof(double);
-        if (bwd)
-            k_log_mean_exp<double, true><<<(unsigned)grid, block, smem, st>>>((double*)out, (const double*)g,
-                                                                               (const double*)x, K, B, cols, slices);
-        else
-            k_log_mean_exp<double, false><<<(unsigned)grid, block, smem, st>>>((double*)out, nullptr,
-                                                                                (const double*)x, K, B, cols, slices);
-    } else {
-        set_last_error_msg("dtype must be ZS_F32 or ZS_F64");
-        return ZS_ERR_DTYPE;
-    }
+            k_log_mean_exp<T, false><<<(unsigned)grid, block, smem, st>>>((T*)out, nullptr, (const T*)x, K, B, cols,
+                                                                           slices);
+    })
     ZS_LAUNCH_CHECK("k_log_mean_exp");
     return ZS_OK;
 }
@@ -439,16 +404,10 @@ int zs_scale_inplace(int dtype, void* buf0, int64_t n0, void* buf1, int64_t n1, 
     if (buf2 && n2 > n) n = n2;
     if (n == 0) return ZS_OK;
     const int grid = grid_for(n / 4 + 1, 256, 8);
-    if (dtype == ZS_F32)
-        launch_pdl(PDL_SCALE, k_scale_inplace<float>, dim3(grid), dim3(256), 0, as_stream(stream), (float*)buf0, n0, (float*)buf1, n1,
-                   (float*)buf2, n2, (const float*)scale_dev);
-    else if (dtype == ZS_F64)
-        launch_pdl(PDL_SCALE, k_scale_inplace<double>, dim3(grid), dim3(256), 0, as_stream(stream), (double*)buf0, n0, (double*)buf1,
-                   n1, (double*)buf2, n2, (const double*)scale_dev);
-    else {
-        set_last_error_msg("dtype must be ZS_F32 or ZS_F64");
-        return ZS_ERR_DTYPE;
-    }
+    ZS_DTYPE_SWITCH(dtype, {
+        launch_pdl(PDL_SCALE, k_scale_inplace<T>, dim3(grid), dim3(256), 0, as_stream(stream), (T*)buf0, n0, (T*)buf1, n1,
+                   (T*)buf2, n2, (const T*)scale_dev);
+    })
     ZS_LAUNCH_CHECK("k_scale_inplace");
     return ZS_OK;
 }
@@ -456,16 +415,10 @@ int zs_scale_inplace(int dtype, void* buf0, int64_t n0, void* buf1, int64_t n1, 
 int zs_combine_sums(int dtype, void* out, const void* a, int64_t na, double scale_a, const void* b, int64_t nb,
                     double scale_b, zs_stream_t stream) {
     ZS_REQUIRE(out && na >= 0 && nb >= 0 && (a || na == 0) && (b || nb == 0), ZS_ERR_ARG);
-    if (dtype == ZS_F32)
-        k_combine_sums<float><<<1, 1024, 0, as_stream(stream)>>>((float*)out, (const float*)a, na, (float)scale_a,
-                                                                   (const float*)b, nb, (float)scale_b);
-    else if (dtype == ZS_F64)
-        k_combine_sums<double><<<1, 1024, 0, as_stream(stream)>>>((double*)out, (const double*)a, na, scale_a,
-                                                                    (const double*)b, nb, scale_b);
-    else {
-        set_last_error_msg("dtype must be ZS_F32 or ZS_F64");
-        return ZS_ERR_DTYPE;
-    }
+    ZS_DTYPE_SWITCH(dtype, {
+        k_combine_sums<T><<<1, 1024, 0, as_stream(stream)>>>((T*)out, (const T*)a, na, (T)scale_a, (const T*)b, nb,
+                                                              (T)scale_b);
+    })
     ZS_LAUNCH_CHECK("k_combine_sums");
     return ZS_OK;
 }
@@ -484,16 +437,11 @@ int zs_reinforce_step(int dtype, void* cost, void* dlogp, void* dlogq, float* mo
                       const void* logp, const void* logq, int64_t N, double decay, double grad_scale,
                       zs_stream_t stream) {
     ZS_REQUIRE(cost && moving_mean && local_step && logp && logq && N >= 1, ZS_ERR_ARG);
-    if (dtype == ZS_F32)
-        k_reinforce<float><<<RF_CLUSTER, RF_THREADS, 0, as_stream(stream)>>>(
-            (float*)cost, (float*)dlogp, (float*)dlogq, moving_mean, local_step, (const float*)logp, (const float*)logq, N,
-            (float)decay, (float)grad_scale);
-    else if (dtype == ZS_F64)
-        k_reinforce<double><<<RF_CLUSTER, RF_THREADS, 0, as_stream(stream)>>>(
-            (double*)cost, (double*)dlogp, (double*)dlogq, moving_mean, local_step, (const double*)logp,
-            (const double*)logq, N, (float)decay, grad_scale);
-    else
-        return ZS_ERR_DTYPE;
+    ZS_DTYPE_SWITCH(dtype, {
+        k_reinforce<T><<<RF_CLUSTER, RF_THREADS, 0, as_stream(stream)>>>((T*)cost, (T*)dlogp, (T*)dlogq, moving_mean,
+                                                                          local_step, (const T*)logp, (const T*)logq, N,
+                                                                          (float)decay, (T)grad_scale);
+    })
     ZS_LAUNCH_CHECK("k_reinforce");
     return ZS_OK;
 }

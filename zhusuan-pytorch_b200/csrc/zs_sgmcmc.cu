@@ -303,15 +303,10 @@ int zs_sgld_step(int dtype, void* w_out, const void* w, const void* g, const voi
     const float lr_f = (float)lr;
     const float std = (float)sqrt((double)lr_f);
     const bool vec = aligned16(w_out) && aligned16(w) && aligned16(g) && aligned16(noise);
-    if (dtype == ZS_F32) {
-        SgldBody<float> b{(float*)w_out, (const float*)w, (const float*)g, (const float*)noise, 0.5f * lr_f, std};
-        return launch_chain<float>(b, n, vec, seed, offset, rng_state, as_stream(stream), "sgld");
-    } else if (dtype == ZS_F64) {
-        SgldBody<double> b{(double*)w_out, (const double*)w, (const double*)g, (const double*)noise, (double)(0.5f * lr_f), std};
-        return launch_chain<double>(b, n, vec, seed, offset, rng_state, as_stream(stream), "sgld");
-    }
-    set_last_error_msg("dtype must be ZS_F32 or ZS_F64");
-    return ZS_ERR_DTYPE;
+    ZS_DTYPE_SWITCH(dtype, {
+        SgldBody<T> b{(T*)w_out, (const T*)w, (const T*)g, (const T*)noise, (T)(0.5f * lr_f), std};
+        return launch_chain<T>(b, n, vec, seed, offset, rng_state, as_stream(stream), "sgld");
+    })
 }
 
 int zs_psgld_step(int dtype, void* w_out, const void* w, void* aux, const void* g, const void* noise_unit, int64_t n,
@@ -320,19 +315,11 @@ int zs_psgld_step(int dtype, void* w_out, const void* w, void* aux, const void* 
     ZS_REQUIRE(w_out && w && aux && g && n >= 0 && lr >= 0, ZS_ERR_ARG);
     const float lr_f = (float)lr;
     const bool vec = aligned16(w_out) && aligned16(w) && aligned16(g) && aligned16(aux) && aligned16(noise_unit);
-    if (dtype == ZS_F32) {
-        PsgldBody<float> b{(float*)w_out, (const float*)w,      (float*)aux,           (const float*)g, (const float*)noise_unit,
-                           (float)decay,   (float)(1.0 - decay),  (float)epsilon,  lr_f,
-                           0.5f * lr_f};
-        return launch_chain<float>(b, n, vec, seed, offset, rng_state, as_stream(stream), "psgld");
-    } else if (dtype == ZS_F64) {
-        PsgldBody<double> b{(double*)w_out, (const double*)w, (double*)aux, (const double*)g, (const double*)noise_unit,
-                            decay,      1.0 - decay,  epsilon,          (double)lr_f,
-                            (double)(0.5f * lr_f)};
-        return launch_chain<double>(b, n, vec, seed, offset, rng_state, as_stream(stream), "psgld");
-    }
-    set_last_error_msg("dtype must be ZS_F32 or ZS_F64");
-    return ZS_ERR_DTYPE;
+    ZS_DTYPE_SWITCH(dtype, {
+        PsgldBody<T> b{(T*)w_out, (const T*)w, (T*)aux, (const T*)g, (const T*)noise_unit,
+                       (T)decay, (T)(1.0 - decay), (T)epsilon, (T)lr_f, (T)(0.5f * lr_f)};
+        return launch_chain<T>(b, n, vec, seed, offset, rng_state, as_stream(stream), "psgld");
+    })
 }
 
 int zs_sghmc_pre(int dtype, void* w_out, const void* w, void* v, const void* v_noise, int64_t n, double lr,
@@ -341,15 +328,10 @@ int zs_sghmc_pre(int dtype, void* w_out, const void* w, void* v, const void* v_n
     if (!resample && !second_order) return ZS_OK;
     const float std = (float)sqrt(lr);
     const bool vec = aligned16(w_out) && aligned16(w) && aligned16(v) && aligned16(v_noise);
-    if (dtype == ZS_F32) {
-        SghmcPreBody<float> b{(float*)w_out, (const float*)w, (float*)v, (const float*)v_noise, std, resample, second_order};
-        return launch_chain<float>(b, n, vec, seed, offset, rng_state, as_stream(stream), "sghmc_pre");
-    } else if (dtype == ZS_F64) {
-        SghmcPreBody<double> b{(double*)w_out, (const double*)w, (double*)v, (const double*)v_noise, std, resample, second_order};
-        return launch_chain<double>(b, n, vec, seed, offset, rng_state, as_stream(stream), "sghmc_pre");
-    }
-    set_last_error_msg("dtype must be ZS_F32 or ZS_F64");
-    return ZS_ERR_DTYPE;
+    ZS_DTYPE_SWITCH(dtype, {
+        SghmcPreBody<T> b{(T*)w_out, (const T*)w, (T*)v, (const T*)v_noise, std, resample, second_order};
+        return launch_chain<T>(b, n, vec, seed, offset, rng_state, as_stream(stream), "sghmc_pre");
+    })
 }
 
 int zs_sghmc_post(int dtype, void* w_out, const void* w, void* v, const void* g, const void* noise, int64_t n,
@@ -360,17 +342,11 @@ int zs_sghmc_post(int dtype, void* w_out, const void* w, void* v, const void* g,
     const float std = (float)sqrt(2.0 * (alpha - beta) * lr);
     const double dh = exp(-0.5 * alpha);
     const bool vec = aligned16(w_out) && aligned16(w) && aligned16(v) && aligned16(g) && aligned16(noise);
-    if (dtype == ZS_F32) {
-        SghmcPostBody<float> b{(float*)w_out, (const float*)w, (float*)v, (const float*)g, (const float*)noise, (float)(1.0 - alpha),
-                               (float)lr, (float)dh, std,             second_order};
-        return launch_chain<float>(b, n, vec, seed, offset, rng_state, as_stream(stream), "sghmc_post");
-    } else if (dtype == ZS_F64) {
-        SghmcPostBody<double> b{(double*)w_out, (const double*)w, (double*)v, (const double*)g, (const double*)noise, 1.0 - alpha,
-                                lr,         dh,         std,              second_order};
-        return launch_chain<double>(b, n, vec, seed, offset, rng_state, as_stream(stream), "sghmc_post");
-    }
-    set_last_error_msg("dtype must be ZS_F32 or ZS_F64");
-    return ZS_ERR_DTYPE;
+    ZS_DTYPE_SWITCH(dtype, {
+        SghmcPostBody<T> b{(T*)w_out, (const T*)w, (T*)v, (const T*)g, (const T*)noise, (T)(1.0 - alpha), (T)lr, (T)dh,
+                           std, second_order};
+        return launch_chain<T>(b, n, vec, seed, offset, rng_state, as_stream(stream), "sghmc_post");
+    })
 }
 
 int zs_sgmcmc_multi_step(int dtype, int algorithm, const zs_chain_tensor* tensors, int n_tensors, double lr, double a,
@@ -380,57 +356,37 @@ int zs_sgmcmc_multi_step(int dtype, int algorithm, const zs_chain_tensor* tensor
     if (n_tensors == 0) return ZS_OK;
     cudaStream_t st = as_stream(stream);
     const float lr_f = (float)lr;  // SGLD / PSGLD: lr is a float32 0-d tensor in the reference (SGLD.py:20)
-    if (dtype != ZS_F32 && dtype != ZS_F64) {
-        set_last_error_msg("dtype must be ZS_F32 or ZS_F64");
-        return ZS_ERR_DTYPE;
-    }
-    const bool f32 = dtype == ZS_F32;
-    switch (algorithm) {
-        case ZS_ALG_SGLD: {
-            const float std = (float)sqrt((double)lr_f);
-            if (f32) {
-                SgldBody<float> p{nullptr, nullptr, nullptr, nullptr, 0.5f * lr_f, std};
-                return launch_chain_multi<float>(p, tensors, n_tensors, seed, offset, rng_state, st, "sgld_multi");
+    ZS_DTYPE_SWITCH(dtype, {
+        switch (algorithm) {
+            case ZS_ALG_SGLD: {
+                const float std = (float)sqrt((double)lr_f);
+                SgldBody<T> p{nullptr, nullptr, nullptr, nullptr, (T)(0.5f * lr_f), std};
+                return launch_chain_multi<T>(p, tensors, n_tensors, seed, offset, rng_state, st, "sgld_multi");
             }
-            SgldBody<double> p{nullptr, nullptr, nullptr, nullptr, (double)(0.5f * lr_f), std};
-            return launch_chain_multi<double>(p, tensors, n_tensors, seed, offset, rng_state, st, "sgld_multi");
-        }
-        case ZS_ALG_PSGLD: {  // a = decay, b = epsilon
-            if (f32) {
-                PsgldBody<float> p{nullptr, nullptr, nullptr, nullptr, nullptr, (float)a, (float)(1.0 - a), (float)b, lr_f,
-                                   0.5f * lr_f};
-                return launch_chain_multi<float>(p, tensors, n_tensors, seed, offset, rng_state, st, "psgld_multi");
+            case ZS_ALG_PSGLD: {  // a = decay, b = epsilon
+                PsgldBody<T> p{nullptr, nullptr, nullptr, nullptr, nullptr, (T)a, (T)(1.0 - a), (T)b, (T)lr_f,
+                               (T)(0.5f * lr_f)};
+                return launch_chain_multi<T>(p, tensors, n_tensors, seed, offset, rng_state, st, "psgld_multi");
             }
-            PsgldBody<double> p{nullptr, nullptr, nullptr, nullptr, nullptr, a, 1.0 - a, b, (double)lr_f,
-                                (double)(0.5f * lr_f)};
-            return launch_chain_multi<double>(p, tensors, n_tensors, seed, offset, rng_state, st, "psgld_multi");
-        }
-        case ZS_ALG_SGHMC_PRE: {
-            if (!resample && !second_order) return ZS_OK;
-            const float std = (float)sqrt(lr);
-            if (f32) {
-                SghmcPreBody<float> p{nullptr, nullptr, nullptr, nullptr, std, resample, second_order};
-                return launch_chain_multi<float>(p, tensors, n_tensors, seed, offset, rng_state, st, "sghmc_pre_multi");
+            case ZS_ALG_SGHMC_PRE: {
+                if (!resample && !second_order) return ZS_OK;
+                const float std = (float)sqrt(lr);
+                SghmcPreBody<T> p{nullptr, nullptr, nullptr, nullptr, std, resample, second_order};
+                return launch_chain_multi<T>(p, tensors, n_tensors, seed, offset, rng_state, st, "sghmc_pre_multi");
             }
-            SghmcPreBody<double> p{nullptr, nullptr, nullptr, nullptr, std, resample, second_order};
-            return launch_chain_multi<double>(p, tensors, n_tensors, seed, offset, rng_state, st, "sghmc_pre_multi");
-        }
-        case ZS_ALG_SGHMC_POST: {  // a = alpha (friction), b = beta (variance estimate)
-            ZS_REQUIRE(a - b >= 0, ZS_ERR_ARG);
-            const float std = (float)sqrt(2.0 * (a - b) * lr);
-            const double dh = exp(-0.5 * a);
-            if (f32) {
-                SghmcPostBody<float> p{nullptr, nullptr, nullptr, nullptr, nullptr, (float)(1.0 - a), (float)lr, (float)dh,
-                                       std, second_order};
-                return launch_chain_multi<float>(p, tensors, n_tensors, seed, offset, rng_state, st, "sghmc_post_multi");
+            case ZS_ALG_SGHMC_POST: {  // a = alpha (friction), b = beta (variance estimate)
+                ZS_REQUIRE(a - b >= 0, ZS_ERR_ARG);
+                const float std = (float)sqrt(2.0 * (a - b) * lr);
+                const double dh = exp(-0.5 * a);
+                SghmcPostBody<T> p{nullptr, nullptr, nullptr, nullptr, nullptr, (T)(1.0 - a), (T)lr, (T)dh, std,
+                                   second_order};
+                return launch_chain_multi<T>(p, tensors, n_tensors, seed, offset, rng_state, st, "sghmc_post_multi");
             }
-            SghmcPostBody<double> p{nullptr, nullptr, nullptr, nullptr, nullptr, 1.0 - a, lr, dh, std, second_order};
-            return launch_chain_multi<double>(p, tensors, n_tensors, seed, offset, rng_state, st, "sghmc_post_multi");
+            default:
+                set_last_error_msg("unknown SG-MCMC algorithm");
+                return ZS_ERR_ARG;
         }
-        default:
-            set_last_error_msg("unknown SG-MCMC algorithm");
-            return ZS_ERR_ARG;
-    }
+    })
 }
 
 }  // extern "C"
